@@ -59,6 +59,10 @@ typedef struct pymfb_ctx pymfb_ctx;
 #define PYMFB_GRAPH_ON   2     /* whenever the loop is replayable (any size) */
 #define PYMFB_OPT_GRAPH 3
 
+/* pass family of pymfb_nndsvd (pymfb_set_option PYMFB_OPT_NNDSVD_PATH, value PYMFB_PATH_*): it has its own, since its
+ * block width (not k) decides what the tensor-core kernels take */
+#define PYMFB_OPT_NNDSVD_PATH 4
+
 /* Library / ABI version (major*1000 + minor). */
 int pymfb_version(void);
 
@@ -196,9 +200,18 @@ int pymfb_gen_h(pymfb_ctx* ctx, uint64_t seed);
  * contractions of the H-update and X H^T passes); the reference's second SVD of max(0, s_i u_i v_i^T) is taken
  * in closed form.  max_iter <= 0 / tol <= 0 / extra_iter < 0 select the defaults (100 sweeps at most, Ritz values
  * settled to 3e-7 relative, then 6 more sweeps).  sigma_out (k doubles, may be null) receives the singular
- * values.  One rank only; k <= 200.
+ * values.  k <= 200.
+ * Column-sharded contexts (world > 1, collective: every rank calls it): X and H are this rank's columns, everything of
+ * length d is replicated.  The fp64 Gram matrix of Q^T X, X Z^T and the column norms of the second SVD are summed over
+ * the ranks on the context's stream; W, sigma_out and iters_done come out bit-identical on every rank, H holds the
+ * rank's columns of the unsharded result.
+ * Pass family: the tensor-core passes (3xTF32) when the shard allows them and d * n_local > 2^24 (>= 2^32 on one GPU
+ * when k > 102, where their block is wider), else the fp32 CUDA-core passes; PYMFB_OPT_NNDSVD_PATH forces either (PYMFB_PATH_TC fails on an unsupported shape).
  */
 int pymfb_nndsvd(pymfb_ctx* ctx, int max_iter, double tol, int extra_iter, int* iters_done, double* sigma_out);
+/* The last pymfb_nndsvd of this context: its pass family (PYMFB_PATH_SIMT / PYMFB_PATH_TC, 0 before the first call)
+ * and the relative change of the leading k Ritz values in its last sweep. */
+int pymfb_nndsvd_info(pymfb_ctx* ctx, int* path, double* change);
 
 /*
  * Run `niter` iterations of the factorize() loop (pymf/nmf.py:182-202): per iteration

@@ -18,6 +18,7 @@ PATH_AUTO, PATH_SIMT, PATH_TC = 0, 1, 2
 OPT_PATH = 1
 OPT_ERR_MODE = 2
 OPT_GRAPH = 3
+OPT_NNDSVD_PATH = 4
 GRAPH_AUTO, GRAPH_OFF, GRAPH_ON = 0, 1, 2
 VARIANT_NMF, VARIANT_SNMF = 0, 1
 ERR_AUTO, ERR_TRACE, ERR_DIRECT = 0, 1, 2
@@ -63,6 +64,7 @@ SIGNATURES = {
                             C.POINTER(C.c_int), C.POINTER(C.c_int)]),
     "pymfb_frobenius": (C.c_int, [_c_ctx, C.POINTER(C.c_double)]),
     "pymfb_nndsvd": (C.c_int, [_c_ctx, C.c_int, C.c_double, C.c_int, C.POINTER(C.c_int), C.POINTER(C.c_double)]),
+    "pymfb_nndsvd_info": (C.c_int, [_c_ctx, C.POINTER(C.c_int), C.POINTER(C.c_double)]),
     "pymfb_enqueue": (C.c_int, [_c_ctx, C.c_int, C.c_uint]),
     "pymfb_sync": (C.c_int, [_c_ctx]),
     "pymfb_stream": (C.c_void_p, [_c_ctx]),

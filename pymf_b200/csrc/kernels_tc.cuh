@@ -397,8 +397,10 @@ struct DoneLag {
 // X/W and H/G stages travel through the same TMA -> split -> MMA rings.
 // warp 0: TMA producer of X, warps 1-2: TMA producers of the operand chunks, warp 3: MMA issuer,
 // warps 4-7: lo split, warps 8..: epilogue.
+// PROD = true (NNDSVD's Z^T = Q^T X, W := Q): the plain product - no G H stages, the epilogue stores C into Hn;
+// Hc, Hs, mapH, mapG, kh_rows, lam, Dp, Dn are not read.
 // ---------------------------------------------------------------------------------------------
-template <int KP>
+template <int KP, bool PROD = false>
 __global__ void __launch_bounds__(HCfg<KP>::THREADS, 1)
 k_h_update_tc(const __grid_constant__ CUtensorMap mapX, const __grid_constant__ CUtensorMap mapW,
               const __grid_constant__ CUtensorMap mapH, const __grid_constant__ CUtensorMap mapG,
@@ -432,7 +434,7 @@ k_h_update_tc(const __grid_constant__ CUtensorMap mapX, const __grid_constant__ 
     const uint32_t tmem_base = *tmem_slot_gen;
 
     const int nd = (d + R1 - 1) / R1;            // stages over the rows of X
-    const int nit = nd + kh_rows / R1;           // + stages over the rows of H (for G H)
+    const int nit = nd + (PROD ? 0 : kh_rows / R1);   // + stages over the rows of H (for G H)
     auto xraw = [&](int s) { return smem_base + s * XSTAGE_BYTES; };
     auto xlo = [&](int s) { return smem_base + Cfg::LO_OFF + s * XSTAGE_BYTES; };
     auto wch = [&](int s) { return smem_base + Cfg::B_OFF + s * Cfg::WSTAGE_BYTES; };
@@ -621,7 +623,13 @@ k_h_update_tc(const __grid_constant__ CUtensorMap mapX, const __grid_constant__ 
                 __syncwarp();
                 if (lane == 0) mbar_arrive(bar.tempty(b));
             }
-            {   // D segment + H update
+            if constexpr (PROD) {
+                const int col = tile * TILE_COLS + q * 32 + lane;
+                if (col < n_loc) {
+#pragma unroll
+                    for (int j = 0; j < Cfg::NJ; ++j) Hn[(int64_t)(jbase + j) * ldh + col] = creg[j];
+                }
+            } else {   // D segment + H update
                 const uint32_t b = g & 1u;
                 mbar_wait_relaxed(bar.tfull(b), (g >> 1) & 1u);
                 tc_fence_after();
@@ -2469,6 +2477,8 @@ template <int KP>
 inline int tc_set_attrs() {
     cudaError_t e = cudaFuncSetAttribute(tc::k_h_update_tc<KP>, cudaFuncAttributeMaxDynamicSharedMemorySize, tc::HCfg<KP>::SMEM_BYTES);
     if (e != cudaSuccess) return 1;
+    e = cudaFuncSetAttribute(tc::k_h_update_tc<KP, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, tc::HCfg<KP>::SMEM_BYTES);
+    if (e != cudaSuccess) return 1;
     e = cudaFuncSetAttribute(tc::k_xht_tc<KP>, cudaFuncAttributeMaxDynamicSharedMemorySize, tc::XCfg<KP>::SMEM_BYTES);
     return e == cudaSuccess ? 0 : 1;
 }
@@ -2512,8 +2522,10 @@ inline void tc_release(TcPlan& p) {
     p.ready = false;
 }
 
+// product = true: a plan for the plain products of NNDSVD (tc_qtx / tc_xzt): SS kernels at every width, SEG_STAGES-stage
+// segments (no ratio whose two chains must match), and always the deterministic combine of the X H^T splits.
 inline int tc_plan(TcPlan& p, int device, int sm_count, int64_t d, int64_t n_loc, int k, int kp, const float* X,
-                   int64_t ldx, int64_t ldh, const float* H0, const float* H1, int64_t xps, int xsh64) {
+                   int64_t ldx, int64_t ldh, const float* H0, const float* H1, int64_t xps, int xsh64, bool product = false) {
     tc_release(p);
     p.device = device; p.sm_count = sm_count; p.d = d; p.n_loc = n_loc; p.k = k; p.kp = kp; p.X = X; p.ldx = ldx; p.ldh = ldh;
     p.xps = xps; p.xsh64 = xsh64; p.xsh = xps != 0 ? xsh64 : tc::kNoPanel;
@@ -2561,7 +2573,7 @@ inline int tc_plan(TcPlan& p, int device, int sm_count, int64_t d, int64_t n_loc
     { const char* e = getenv("PYMFB_TS_RS"); p.ts_rs = e ? atoi(e) : (kp == 32 ? 64 : 1); }
     {
         const char* force_ss = getenv("PYMFB_TC_FORCE_SS");
-        p.use_ts = kp <= 64 && !(force_ss && force_ss[0] == '1');
+        p.use_ts = !product && kp <= 64 && !(force_ss && force_ss[0] == '1');
         if (p.use_ts && (kp == 32 ? ts_set_attrs<32>() : ts_set_attrs<64>())) { p.err = "cudaFuncSetAttribute (TS kernels) failed"; return 1; }
     }
     int rc = p.kpb == 32 ? tc_set_attrs<32>() : p.kpb == 64 ? tc_set_attrs<64>() : p.kpb == 96 ? tc_set_attrs<96>() : tc_set_attrs<128>();
@@ -2582,7 +2594,7 @@ inline int tc_plan(TcPlan& p, int device, int sm_count, int64_t d, int64_t n_loc
         const char* e = getenv("PYMFB_SEG_C");
         const char* ce = getenv("PYMFB_CENTER");
         p.center = p.use_ts && !(ce && ce[0] == '0');
-        p.seg_c = (e && atoi(e) > 0) ? atoi(e) : (p.center ? tc::SEG_STAGES : std::max(1, kp / tc::R1));
+        p.seg_c = (e && atoi(e) > 0) ? atoi(e) : ((p.center || product) ? tc::SEG_STAGES : std::max(1, kp / tc::R1));
         if (p.center) {
             if (cudaMalloc(&p.xsum, (size_t)n_loc * sizeof(float)) != cudaSuccess) { p.err = "cudaMalloc xsum failed"; return 1; }
             if (cudaMalloc(&p.wmean, (size_t)(2 + tc::CM_SPLITS) * kp * sizeof(float)) != cudaSuccess) { p.err = "cudaMalloc wmean failed"; return 1; }
@@ -2632,7 +2644,7 @@ inline int tc_plan(TcPlan& p, int device, int sm_count, int64_t d, int64_t n_loc
         p.x_splits = p.x_tasks / p.x_rb;
         const size_t bytes = ((size_t)p.x_splits * d * kp + (size_t)p.hh_tasks * kp * kp) * sizeof(float);
         const char* e = getenv("PYMFB_DETERMINISTIC");
-        const bool want = e ? e[0] == '1' : bytes <= ((size_t)1 << 30);
+        const bool want = product || (e ? e[0] == '1' : bytes <= ((size_t)1 << 30));
         if (want) {
             if (cudaMalloc(&p.xpart, bytes) != cudaSuccess) { p.err = "cudaMalloc X.H^T partial copies failed"; return 1; }
             p.xpartB = p.xpart + (size_t)p.x_splits * d * kp;
@@ -2794,6 +2806,47 @@ inline int tc_xht(TcPlan& p, const DevState* st, const float* Hc, float* P, cuda
     }
     *launches += 2 * p.nblk;
     sum_copies();
+    return cudaGetLastError() == cudaSuccess ? 0 : 1;
+}
+
+// ---- the two products of an NNDSVD sweep on a product plan (tc_plan(..., product = true)): kp = b' bases, Hbuf = {Zt, Zt2}
+template <int KP>
+inline void tc_launch_qtx(TcPlan& p, const DevState* st, float* Zt, cudaStream_t stream) {
+    const int grid = std::min(p.h_tiles, p.sm_count);
+    for (int b = 0; b < p.nblk; ++b)      // mapH / mapG are never read in product mode: any valid map will do
+        tc::k_h_update_tc<KP, true><<<grid, tc::HCfg<KP>::THREADS, tc::HCfg<KP>::SMEM_BYTES, stream>>>(
+            p.mapX_h, p.mapW_b[b], p.mapX_h, p.mapW_b[b], st, nullptr, Zt + (size_t)b * p.kpb * p.ldh, nullptr,
+            p.ldh, (int)p.d, (int)p.n_loc, p.h_tiles, nullptr, 0, p.seg_c, 0.f, nullptr, nullptr, p.xsh, p.ss_pf);
+}
+// Zt (kp x ldh) = Q^T X, Q: d x kp row-major
+inline int tc_qtx(TcPlan& p, const DevState* st, const float* Q, float* Zt, cudaStream_t stream, int64_t* launches) {
+    const int64_t nw = p.d * p.kpb;
+    for (int b = 0; b < p.nblk; ++b)
+        tc::k_split_hilo<<<(unsigned)((nw + 255) / 256), 256, 0, stream>>>(st, Q, p.d, p.kp, b * p.kpb, p.kpb, p.Wsplit + (size_t)b * p.d * 2 * p.kpb);
+    switch (p.kpb) {
+        case 32: tc_launch_qtx<32>(p, st, Zt, stream); break;
+        case 64: tc_launch_qtx<64>(p, st, Zt, stream); break;
+        case 96: tc_launch_qtx<96>(p, st, Zt, stream); break;
+        default: tc_launch_qtx<128>(p, st, Zt, stream); break;
+    }
+    *launches += 2 * p.nblk;
+    return cudaGetLastError() == cudaSuccess ? 0 : 1;
+}
+// Y (d x kp row-major) = X Zt2^T with Zt2 = Hbuf[1]: the X H^T pass, its column splits summed in split order
+inline int tc_xzt(TcPlan& p, const DevState* st, float* Y, cudaStream_t stream, int64_t* launches) {
+    for (int b = 0; b < p.nblk; ++b)
+        tc::k_split_rows<<<4 * p.sm_count, 256, 0, stream>>>(st, p.Hbuf[1] + (size_t)b * p.kpb * p.ldh, p.kpb, p.ldh,
+                                                            p.Hs[1] + (size_t)b * 2 * p.kpb * p.ldh);
+    switch (p.kpb) {
+        case 32: tc_launch_x<32>(p, st, 1, Y, stream); break;
+        case 64: tc_launch_x<64>(p, st, 1, Y, stream); break;
+        case 96: tc_launch_x<96>(p, st, 1, Y, stream); break;
+        default: tc_launch_x<128>(p, st, 1, Y, stream); break;
+    }
+    const int64_t na = p.d * p.kp;
+    tc::k_sum_copies<<<(unsigned)std::min<int64_t>((na / 4 + 255) / 256, 8 * p.sm_count), 256, 0, stream>>>(
+        st, p.xpart, p.x_splits, na, Y, nullptr, 0, 0, nullptr);
+    *launches += 2 * p.nblk + 1;
     return cudaGetLastError() == cudaSuccess ? 0 : 1;
 }
 

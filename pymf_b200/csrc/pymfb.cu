@@ -212,7 +212,10 @@ struct pymfb_ctx {
     int world = 1, rank = 0;
 
     int64_t launches = 0;
-    float* xpart_simt = nullptr;          // SIMT X H^T pass: copies of [A | B] for the deterministic combine of the column splits
+    int nndsvd_path_opt = PYMFB_PATH_AUTO;
+    int nndsvd_path = 0;                  // pass family of the last pymfb_nndsvd (PYMFB_PATH_SIMT / _TC), 0 = none yet
+    double nndsvd_change = 0.0;           // its last sweep-to-sweep change of the Ritz values (pymfb_nndsvd_info)
+    float* xpart_simt = nullptr;         // SIMT X H^T pass: copies of [A | B] for the deterministic combine of the column splits
     bool deterministic_simt = true;       // PYMFB_DETERMINISTIC=0: fp32 atomics
     bool uw_smem_set = false;      // k_update_w's dynamic shared memory attribute raised (k > 1536)
     bool last_upload_pinned = false;
@@ -797,6 +800,11 @@ int pymfb_set_option(pymfb_ctx* c, int option, int64_t value) {
         if (value < 0 || value > 2) return fail("bad path option %lld", (long long)value);
         c->path_opt = (int)value;
         if (c->X) { CK(resolve_path(c)); if (c->path == PYMFB_PATH_TC) CK(plan_tc(c)); c->g_valid = false; }
+        return 0;
+    }
+    if (option == PYMFB_OPT_NNDSVD_PATH) {
+        if (value < 0 || value > 2) return fail("bad NNDSVD path option %lld", (long long)value);
+        c->nndsvd_path_opt = (int)value;
         return 0;
     }
     if (option == PYMFB_OPT_ERR_MODE) {
@@ -1446,22 +1454,42 @@ int pymfb_gen_h(pymfb_ctx* c, uint64_t seed) {
 }
 
 // ---- NNDSVD initialisation (pymf/nndsvd.py:79-108), kernels_svd.cuh -----------------------------
+// The tensor-core passes by default only beyond the graph-replay sizes, the rule of the one-pass NMF kernel: below it the
+// CUDA-core passes keep the results of the tested shapes as they were.  Where the tensor-core width enlarges the block
+// (b = 160..224 -> 256, one GPU) the b x b work of the wider block outweighs the faster passes up to much larger X
+// (measured, DESIGN 5.7: 16384 x 131072 k=128 0.81x, 8192 x 524288 k=128 1.22x).
+static const double kNndsvdTcMinWork = 16777216.0;     // d * n_local
+static const double kNndsvdTcMinWorkWider = 4294967296.0;
 int pymfb_nndsvd(pymfb_ctx* c, int max_iter, double tol, int extra_iter, int* iters_done, double* sigma_out) {
     if (!c) return fail("null context");
     if (!c->X) return fail("no data bound: call pymfb_bind_x / pymfb_upload_x / pymfb_gen_x first");
-    if (c->world > 1) return fail("pymfb_nndsvd runs on one rank (initialise there and broadcast W; H rows follow from the shards)");
+    if (c->world > 1 && !c->comm) return fail("pymfb_nndsvd: world = %d but no communicator is attached", c->world);
     if (max_iter < 1) max_iter = 100;
-    if (!(tol > 0.0)) tol = 3e-7;
     if (extra_iter < 0) extra_iter = 6;
     CU(cudaSetDevice(c->device));
     const int k = c->k;
-    const int b = (int)round_up(k + std::max(8, k / 4), 32);          // block of the subspace iteration (oversampled)
-    if (b > 256) return fail("NNDSVD supports k <= 200 (subspace block %d > 256)", b);
+    const int b_simt = (int)round_up(k + std::max(8, k / 4), 32);     // block of the subspace iteration (oversampled)
+    if (b_simt > 256) return fail("NNDSVD supports k <= 200 (subspace block %d > 256)", b_simt);
+    const int b_tc = b_simt <= 128 ? b_simt : 256;                      // a width the SS kernels take (256: two 128-wide blocks)
     const int64_t d = c->d, n = c->n_loc, ldz = c->ldh;
-    const int b_real = (int)std::min<int64_t>(b, std::min(d, n));
+    std::string why;
+    const bool tc_ok = tc_supported(d, n, b_tc, c->ldx, c->X, &why);
+    const double dn = (double)d * (double)n;
+    bool use_tc = tc_ok && dn > kNndsvdTcMinWork && (b_tc == b_simt || c->world > 1 || dn >= kNndsvdTcMinWorkWider);
+    if (c->nndsvd_path_opt == PYMFB_PATH_SIMT) use_tc = false;
+    if (c->nndsvd_path_opt == PYMFB_PATH_TC) {
+        if (!tc_ok) return fail("tcgen05 path not available for NNDSVD on this shape: %s", why.c_str());
+        use_tc = true;
+    }
+    // Shards pick their pass family on their own (a narrow one stays on the CUDA cores), so a sharded run iterates the
+    // tensor-core width on every rank: the collectives below need the same block everywhere.  Extra vectors only oversample.
+    const int b = (use_tc || c->world > 1) ? b_tc : b_simt;
+    if (!(tol > 0.0)) tol = 3e-7;
+    const int b_real = (int)std::min<int64_t>(b, std::min(d, c->n_glob));
     cudaStream_t s = c->stream;
     float *Q = nullptr, *Y = nullptr, *Zt = nullptr, *Zt2 = nullptr, *Rm = nullptr, *Rt = nullptr, *Ct = nullptr, *Ppart = nullptr;
     double *gpart = nullptr, *Tm = nullptr, *work = nullptr, *vals = nullptr, *norms = nullptr;
+    TcPlan tp;                                                  // Q^T X / X Z^T on the tensor cores (use_tc), freed below
     // X Z^T launches: column splits combined deterministically (k_xht_simt)
     const int64_t rowblocks = (d + 127) / 128, kblocks = b / 32, chunks = (n + XHT_CK - 1) / XHT_CK;
     int64_t want = std::min<int64_t>(chunks, std::max<int64_t>(1, (4LL * c->sm_count) / (rowblocks * kblocks)));
@@ -1476,6 +1504,7 @@ int pymfb_nndsvd(pymfb_ctx* c, int max_iter, double tol, int extra_iter, int* it
         cudaStreamSynchronize(s);
         cudaFree(Q); cudaFree(Y); cudaFree(Zt); cudaFree(Zt2); cudaFree(Rm); cudaFree(Rt); cudaFree(Ct); cudaFree(Ppart);
         cudaFree(gpart); cudaFree(Tm); cudaFree(work); cudaFree(vals); cudaFree(norms);
+        tc_release(tp);
     };
 #define SV(call)                                                                                   \
     do {                                                                                           \
@@ -1486,6 +1515,10 @@ int pymfb_nndsvd(pymfb_ctx* c, int max_iter, double tol, int extra_iter, int* it
             return rc;                                                                             \
         }                                                                                          \
     } while (0)
+#define SK(call)                                                                                   \
+    do {                                                                                           \
+        if ((rc = (call)) != 0) { cleanup(); return rc; }                                          \
+    } while (0)
     SV(cudaMalloc(&Q, (size_t)d * b * 4)); SV(cudaMalloc(&Y, (size_t)d * b * 4));
     SV(cudaMalloc(&Zt, (size_t)b * ldz * 4)); SV(cudaMalloc(&Zt2, (size_t)b * ldz * 4));
     SV(cudaMemsetAsync(Zt, 0, (size_t)b * ldz * 4, s)); SV(cudaMemsetAsync(Zt2, 0, (size_t)b * ldz * 4, s));
@@ -1493,7 +1526,18 @@ int pymfb_nndsvd(pymfb_ctx* c, int max_iter, double tol, int extra_iter, int* it
     SV(cudaMalloc(&gpart, (size_t)std::max(gsplit_n, gsplit_d) * b * b * 8)); SV(cudaMalloc(&Tm, (size_t)b * b * 8));
     SV(cudaMalloc(&work, (size_t)2 * b * b * 8)); SV(cudaMalloc(&vals, (size_t)b * 8)); SV(cudaMalloc(&norms, (size_t)4 * b * 8));
     // (a non-null Ppart selects k_xht_simt's overwrite mode, also for a single split)
-    SV(cudaMalloc(&Ppart, ns > 1 ? (size_t)ns * d * b * 4 : 16));
+    SV(cudaMalloc(&Ppart, ns > 1 && !use_tc ? (size_t)ns * d * b * 4 : 16));
+    if (use_tc && tc_plan(tp, c->device, c->sm_count, d, n, b, b, c->X, c->ldx, ldz, Zt, Zt2, c->xps, c->xsh, true)) {
+        rc = fail("tcgen05 plan for NNDSVD failed: %s", tp.err.c_str());
+        cleanup();
+        return rc;
+    }
+    // in-place sum over the ranks on the context's stream (replicated quantities: the same on every rank afterwards)
+    auto rank_sum = [&](void* buf, size_t count, int dtype) -> int {
+        if (c->world == 1) return 0;
+        const int r = g_nccl.AllReduce(buf, buf, count, dtype, kNcclSum, c->comm, s);
+        return r ? fail("NNDSVD ncclAllReduce -> nccl error %d (%s)", r, g_nccl.GetErrorString ? g_nccl.GetErrorString(r) : "?") : 0;
+    };
     // G = A^T A (by_rows = 0, A: len x b) or A A^T (by_rows = 1, A: b x len) in fp64 -> Tm
     auto gram = [&](const float* A, int64_t ld, int64_t len, int by_rows) {
         const int sp = by_rows ? gsplit_n : gsplit_d;
@@ -1522,55 +1566,86 @@ int pymfb_nndsvd(pymfb_ctx* c, int max_iter, double tol, int extra_iter, int* it
         c->launches += 1;
         right_mul(A, Ct, Out);
     };
-    auto rayleigh_ritz = [&]() {                                  // Zt = Q^T X; eigh(Zt Zt^T) -> vals, Rm, Rt
-        left_mul_t(Q, b, d, c->X, c->ldx, Zt);
+    auto rayleigh_ritz = [&]() -> int {                          // Zt = Q^T X; eigh(sum over ranks of Zt Zt^T) -> vals, Rm, Rt
+        if (use_tc) {
+            if (tc_qtx(tp, c->st, Q, Zt, s, &c->launches)) return fail("tcgen05 Q^T X launch failed: %s", cudaGetErrorString(cudaGetLastError()));
+        } else {
+            left_mul_t(Q, b, d, c->X, c->ldx, Zt);
+        }
         gram(Zt, ldz, n, 1);
+        CK(rank_sum(Tm, (size_t)b * b, kNcclFloat64));
         svd::k_jacobi_eigh_f64<<<1, 256, 0, s>>>(Tm, b, work, vals, Rm, Rt);
         c->launches += 1;
+        return 0;
+    };
+    auto x_zt = [&]() -> int {                                   // Y = sum over ranks of X Zt2^T
+        if (use_tc) {
+            if (tc_xzt(tp, c->st, Y, s, &c->launches)) return fail("tcgen05 X Z^T launch failed: %s", cudaGetErrorString(cudaGetLastError()));
+        } else {
+            k_xht_simt<32><<<dim3((unsigned)rowblocks, ns, (unsigned)kblocks), SIMT_THREADS, 0, s>>>(
+                c->st, c->X, c->ldx, d, Zt2, ldz, n, cps, Y, b, (int)rowblocks, 0, nullptr, Ppart, d * b, c->xps, c->xsh);
+            if (ns > 1)
+                tc::k_sum_copies<<<grid_for(d * b / 4, 256, 4 * c->sm_count), 256, 0, s>>>(c->st, Ppart, (int)ns, d * b, Y, nullptr, 0, 0, nullptr);
+            c->launches += 2;
+        }
+        return rank_sum(Y, (size_t)d * b, kNcclFloat32);
     };
     svd::k_svd_seed<<<(unsigned)((d * b + 255) / 256), 256, 0, s>>>(Y, d, b, b_real, 0x5EEDull);
     c->launches += 1;
     orthonormalise(Y, Q);
     std::vector<double> ev(b, 0.0), prev(b, 0.0);
     int it = 0, settled = -1;
+    double worst = 0.0;
     for (; it < max_iter; ++it) {
-        rayleigh_ritz();
+        SK(rayleigh_ritz());
         left_mul_t(Rm, b, b, Zt, ldz, Zt2);                      // rows of Zt2: (Ritz vector)^T X
-        k_xht_simt<32><<<dim3((unsigned)rowblocks, ns, (unsigned)kblocks), SIMT_THREADS, 0, s>>>(
-            c->st, c->X, c->ldx, d, Zt2, ldz, n, cps, Y, b, (int)rowblocks, 0, nullptr, Ppart, d * b, c->xps, c->xsh);
-        if (ns > 1)
-            tc::k_sum_copies<<<grid_for(d * b / 4, 256, 4 * c->sm_count), 256, 0, s>>>(c->st, Ppart, (int)ns, d * b, Y, nullptr, 0, 0, nullptr);
-        c->launches += 2;
+        SK(x_zt());
         orthonormalise(Y, Q);                                    // Y = X X^T (Ritz vectors) -> next Q
         SV(cudaGetLastError());
         SV(cudaMemcpyAsync(ev.data(), vals, (size_t)b * 8, cudaMemcpyDeviceToHost, s));
         SV(cudaStreamSynchronize(s));
-        double worst = 0.0;
+        worst = 0.0;
         for (int i = 0; i < k; ++i) worst = std::max(worst, std::fabs(ev[i] - prev[i]) / std::max(std::fabs(ev[i]), 1e-300));
         prev = ev;
         if (settled < 0 && it > 0 && worst < tol) settled = it;
         if (settled >= 0 && it >= settled + extra_iter) { ++it; break; }
     }
     // final extraction with the converged basis: U = Q R, S = sqrt(vals), S V^T = R^T Q^T X
-    rayleigh_ritz();
+    SK(rayleigh_ritz());
     right_mul(Q, Rt, Y);                                         // U -> Y
     left_mul_t(Rm, b, b, Zt, ldz, Zt2);                          // S V^T -> Zt2
     svd::k_posneg_norms<<<dim3((unsigned)k, 2), 256, 0, s>>>(Y, b, d, Zt2, ldz, n, vals, norms);
+    c->launches += 1;
+    if (c->world > 1) {
+        // |u+|, |u-| (entries 0, 1 of each basis) are the same on every rank: rank 0 contributes them, the others 0 (exact),
+        // so that one sum gives |v+|^2, |v-|^2 over all columns and leaves the u norms as they are
+        if (c->rank != 0) SV(cudaMemset2DAsync(norms, 4 * sizeof(double), 0, 2 * sizeof(double), (size_t)k, s));
+        SK(rank_sum(norms, (size_t)4 * k, kNcclFloat64));
+    }
     SV(cudaMemsetAsync(c->W[c->wcur], 0, (size_t)d * c->kp * sizeof(float), s));
     SV(cudaMemsetAsync(c->H[c->hcur], 0, (size_t)c->kp * c->ldh * sizeof(float), s));
     svd::k_nndsvd_fill<<<dim3((unsigned)std::min<int64_t>((d + n + 255) / 256, 8 * c->sm_count), (unsigned)k), 256, 0, s>>>(
         Y, b, d, Zt2, ldz, n, vals, norms, k, c->W[c->wcur], c->kp, c->H[c->hcur], c->ldh);
-    c->launches += 2;
+    c->launches += 1;
     SV(cudaGetLastError());
     SV(cudaMemcpyAsync(ev.data(), vals, (size_t)b * 8, cudaMemcpyDeviceToHost, s));
     SV(cudaStreamSynchronize(s));
 #undef SV
+#undef SK
     cleanup();
     if (sigma_out) for (int i = 0; i < k; ++i) sigma_out[i] = std::sqrt(std::max(ev[i], 0.0));
     if (iters_done) *iters_done = it;
+    c->nndsvd_path = use_tc ? PYMFB_PATH_TC : PYMFB_PATH_SIMT;
+    c->nndsvd_change = worst;
     c->w_set = c->h_set = true;
     c->g_valid = false; c->ab_valid = false; c->p_zeroed = false;
     c->tc.hs_valid[0] = c->tc.hs_valid[1] = false;
+    return 0;
+}
+int pymfb_nndsvd_info(pymfb_ctx* c, int* path, double* change) {
+    if (!c) return fail("null context");
+    if (path) *path = c->nndsvd_path;
+    if (change) *change = c->nndsvd_change;
     return 0;
 }
 

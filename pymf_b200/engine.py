@@ -102,6 +102,11 @@ class Engine(object):
         code = {"auto": _lib.PATH_AUTO, "simt": _lib.PATH_SIMT, "tc": _lib.PATH_TC}.get(path, path)
         _lib.check(self._lib.pymfb_set_option(self._ctx, _lib.OPT_PATH, int(code)))
 
+    def set_nndsvd_path(self, path):
+        """'auto' | 'simt' | 'tc': pass family of nndsvd()."""
+        code = {"auto": _lib.PATH_AUTO, "simt": _lib.PATH_SIMT, "tc": _lib.PATH_TC}.get(path, path)
+        _lib.check(self._lib.pymfb_set_option(self._ctx, _lib.OPT_NNDSVD_PATH, int(code)))
+
     def set_err_mode(self, mode):
         """'auto' | 'trace' (trace identity, no extra pass) | 'direct' (||X - WH|| as written)."""
         code = {"auto": _lib.ERR_AUTO, "trace": _lib.ERR_TRACE, "direct": _lib.ERR_DIRECT}.get(mode, mode)
@@ -267,6 +272,10 @@ class Engine(object):
         it = C.c_int(0)
         _lib.check(self._lib.pymfb_nndsvd(self._ctx, int(max_iter), float(tol), int(extra_iter), C.byref(it),
                                           sig.ctypes.data_as(C.POINTER(C.c_double))))
+        path, change = C.c_int(0), C.c_double(0.0)
+        _lib.check(self._lib.pymfb_nndsvd_info(self._ctx, C.byref(path), C.byref(change)))
+        self.nndsvd_path = {_lib.PATH_SIMT: "simt", _lib.PATH_TC: "tc"}.get(path.value, "?")   # pass family it ran
+        self.nndsvd_change = change.value         # relative change of the Ritz values in its last sweep
         return sig, it.value
 
     def frobenius(self):

@@ -20,12 +20,22 @@ class NNDSVD(NMF):
 
     Drop-in for ``pymf.nndsvd.NNDSVD``: after ``factorize()``, ``W`` (data_dimension x num_bases) and
     ``H`` (num_bases x num_samples) hold the non-negative double SVD factors and ``ferr`` the Frobenius
-    error ``|data - W*H|``.  ``singular_values`` (extra) holds the leading singular values of ``data``.
-    Single GPU; ``num_bases`` <= 200.
+    error ``|data - W*H|``.  ``singular_values`` (extra) holds the leading singular values of ``data``,
+    ``svd_sweeps`` the subspace-iteration sweeps it took and ``svd_path`` the kernel family of its passes over
+    ``data`` ("simt": fp32 CUDA cores, "tc": 3xTF32 tensor cores; ``path=`` forces one).  ``num_bases`` <= 200.
+
+    With ``process_group`` (column-sharded ``data``, as for ``NMF``) every rank gets the same ``W``,
+    ``singular_values`` and ``svd_sweeps`` and its own columns of ``H``: the blocks of what the unsharded data gives,
+    ready for a sharded ``NMF`` on the same shards.
 
     >>> init = NNDSVD(data, num_bases=8); init.factorize()
     >>> mdl = NMF(data, num_bases=8); mdl.W = init.W; mdl.H = init.H; mdl.factorize(niter=50)
     """
+
+    def __init__(self, data, num_bases=4, **kw):
+        # path= selects the family of the SVD passes; the engine's own NMF kernels (the error pass) keep their default
+        self._svd_path_opt = kw.pop("path", None) or "auto"
+        super(NNDSVD, self).__init__(data, num_bases, **kw)
 
     @staticmethod
     def _native_hooks():
@@ -35,16 +45,16 @@ class NNDSVD(NMF):
         self.W = np.zeros((self._data_dimension, self._num_bases))
 
     def init_h(self):                                                    # pymf/nndsvd.py:73-74
-        self.H = np.zeros((self._num_bases, self._num_samples))
+        self.H = np.zeros((self._num_bases, self._n_local))              # this rank's columns (all of them unsharded)
 
     def update_h(self):                                                  # pymf/nndsvd.py:76-77
         pass
 
     def update_w(self):                                                  # pymf/nndsvd.py:79-108
-        if self._world > 1:
-            raise NotImplementedError("NNDSVD runs on one GPU: initialise there and hand W / H to the sharded NMF")
         eng = self._sync_to_device()
+        eng.set_nndsvd_path(self._svd_path_opt)
         self.singular_values, self.svd_sweeps = eng.nndsvd()
+        self.svd_path = eng.nndsvd_path
         self._mark_device_newer("W")
         self._mark_device_newer("H")
 
