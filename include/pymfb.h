@@ -42,6 +42,8 @@ typedef struct pymfb_ctx pymfb_ctx;
 #define PYMFB_PATH_AUTO 0      /* tcgen05 kernels when the shape allows, else SIMT */
 #define PYMFB_PATH_SIMT 1      /* fp32 CUDA-core kernels (exact fp32 FMA) */
 #define PYMFB_PATH_TC   2      /* tcgen05 3xTF32 kernels; error if the shape is unsupported */
+#define PYMFB_PATH_SPARSE 3    /* reported only: the sparse passes of a context holding a CSC X (pymfb_upload_x_csc);
+                                  setting PYMFB_PATH_SIMT / _TC on such a context is an error */
 
 #define PYMFB_OPT_PATH 1
 
@@ -145,6 +147,20 @@ int pymfb_comm_destroy(void* comm);
 int pymfb_bind_x(pymfb_ctx* ctx, const float* x_dev, int64_t ld);
 int pymfb_upload_x(pymfb_ctx* ctx, const void* x_host, int dtype, int64_t ld);
 int pymfb_gen_x(pymfb_ctx* ctx, uint64_t seed);
+
+/*
+ * Sparse X in compressed sparse column form: colptr (n_local + 1 entries), rowidx and values (nnz entries each, values
+ * fp32 or fp64 by dtype, cast to fp32 on the device).  The arrays are validated on the device before any kernel indexes
+ * with them - colptr[0] == 0, colptr non-decreasing, colptr[n_local] == nnz, 0 <= row < d, rows strictly increasing
+ * within a column - and a malformed matrix returns non-zero with the broken rules in pymfb_last_error().
+ * On success the sparse X becomes current: the dense X and the tensor-core plan are freed, pymfb_active_path reports
+ * PYMFB_PATH_SPARSE, and the loop (pymfb_run, pymfb_frobenius, pymfb_enqueue) runs the sparse passes: the H update over
+ * the CSC, X H^T over a column-panel CSR built on the device.  A later pymfb_upload_x / pymfb_bind_x / pymfb_gen_x
+ * switches back to dense data.  pymfb_nndsvd on a sparse context is an error.  nnz < 2^31.
+ * PYMFB_SPARSE_PANEL=<columns> (environment, read at each upload) forces the CSR panel width.
+ */
+int pymfb_upload_x_csc(pymfb_ctx* ctx, const int64_t* colptr /* n_local+1 */, const int32_t* rowidx,
+                       const void* values, int dtype, int64_t nnz);
 
 /*
  * Ingest fast path (SURVEY 8f rank 2, the step before the hot path).  pymfb_upload_x looks at
@@ -255,7 +271,7 @@ int64_t pymfb_launch_count(pymfb_ctx* ctx);
  * pymfb_launch_count). */
 int64_t pymfb_graph_replays(pymfb_ctx* ctx);
 
-/* Which path the context resolved to for its shape: PYMFB_PATH_SIMT or PYMFB_PATH_TC. */
+/* Which path the context resolved to for its data: PYMFB_PATH_SIMT, PYMFB_PATH_TC or PYMFB_PATH_SPARSE. */
 int pymfb_active_path(pymfb_ctx* ctx);
 
 /* Write a buffer larger than L2 (flush between timed iterations of small problems). */

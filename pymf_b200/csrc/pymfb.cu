@@ -41,6 +41,9 @@
 #include "kernels_tc2.cuh"
 #include "kernels_fused.cuh"
 #include "kernels_svd.cuh"
+#include "kernels_sparse.cuh"
+
+#include <cub/device/device_radix_sort.cuh>
 
 using namespace pymfb;
 
@@ -145,11 +148,29 @@ static int nccl_load() {
 // ------------------------------------------------------------------------------------------
 // Host-side scheduling state that decides which kernels an iteration launches and on which buffers.
 struct LoopState {
-    int wcur, hcur; bool ab, g, xx, hs0, hs1;
+    int wcur, hcur; bool ab, g, xx, hs0, hs1; int ht;
     bool operator==(const LoopState& o) const {
-        return wcur == o.wcur && hcur == o.hcur && ab == o.ab && g == o.g && xx == o.xx && hs0 == o.hs0 && hs1 == o.hs1;
+        return wcur == o.wcur && hcur == o.hcur && ab == o.ab && g == o.g && xx == o.xx && hs0 == o.hs0 && hs1 == o.hs1 &&
+               ht == o.ht;
     }
 };
+
+// Sparse X on the device (kernels_sparse.cuh): CSC and the column-panel CSR built from it.
+struct SparseX {
+    int64_t nnz = 0;
+    int64_t* colptr = nullptr;     // n_local + 1
+    int32_t* rowidx = nullptr;     // nnz
+    float* vals = nullptr;         // nnz rounded up to a multiple of 4, zero-padded
+    int64_t pw = 0;                // columns per CSR panel
+    int npanels = 0;
+    int64_t* rowptr = nullptr;     // npanels * d + 1
+    int32_t* ccol = nullptr;       // nnz: column of each CSR entry
+    float* cval = nullptr;         // nnz
+};
+static void sparse_free(SparseX& s) {
+    cudaFree(s.colptr); cudaFree(s.rowidx); cudaFree(s.vals); cudaFree(s.rowptr); cudaFree(s.ccol); cudaFree(s.cval);
+    s = SparseX();
+}
 
 struct pymfb_ctx {
     int device = 0;
@@ -245,11 +266,21 @@ struct pymfb_ctx {
     int graph_opt = PYMFB_GRAPH_AUTO;
     cudaGraphExec_t graph_exec = nullptr;
     unsigned graph_key = 0;
-    LoopState graph_state = {0, 0, false, false, false, false, false};
+    LoopState graph_state = {0, 0, false, false, false, false, false, -1};
     int64_t graph_launches = 0, graph_replays = 0;
 
     // BNMF penalty (pymf/bnmf.py:70-90): weights of the current iteration and their growth per H update; 0 = NMF
     double lam_w = 0.0, lam_h = 0.0, inc_w = 1.0, inc_h = 1.0;
+
+    // sparse X (pymfb_upload_x_csc): current instead of X while `sparse`
+    bool sparse = false;
+    SparseX sx;
+    float* Ht = nullptr;           // n_loc x kp: H^T of H[ht_of] (-1: of neither buffer), gathered by the X H^T pass
+    int ht_of = -1;
+    float* GH = nullptr;           // kp x ldh: G H for the sparse H update (NMF / BNMF)
+    float* hh_part = nullptr;      // hh_splits x kp x kp: row-split partials of H H^T = (H^T)^T H^T
+    int hh_splits = 1;
+    int64_t hh_rows_per_split = 0;
 
     // per-kernel timing (CUDA events on the launch stream)
     bool timing = false;
@@ -302,6 +333,12 @@ static int timing_end(pymfb_ctx* c, int which, cudaEvent_t e0, cudaEvent_t e1) {
 // kernel scheduling helpers
 // ------------------------------------------------------------------------------------------
 static int resolve_path(pymfb_ctx* c) {
+    if (c->sparse) {
+        if (c->path_opt == PYMFB_PATH_SIMT || c->path_opt == PYMFB_PATH_TC)
+            return fail("sparse data runs on its own passes: the dense kernel families (path simt / tc) do not apply");
+        c->path = PYMFB_PATH_SPARSE;
+        return 0;
+    }
     std::string why;
     bool ok = tc_supported(c->d, c->n_loc, c->kp, c->ldx, c->X, &why);
     if (c->path_opt == PYMFB_PATH_SIMT) { c->path = PYMFB_PATH_SIMT; return 0; }
@@ -365,6 +402,72 @@ static int launch_update_w(pymfb_ctx* c) {
     return 0;
 }
 
+// k block of the sparse passes: the widest of 128 / 64 / 32 / 16 that divides kp
+static int sparse_kblk(int kp) { return kp % 128 == 0 ? 128 : kp % 64 == 0 ? 64 : kp % 32 == 0 ? 32 : 16; }
+
+// Sparse H update: D = G H (G+ H, G- H for Semi-NMF), then H[hcur^1] and Ht from the CSC
+static int launch_h_update_sparse(pymfb_ctx* c, bool snmf) {
+    const float* Hc = c->H[c->hcur];
+    dim3 gg((unsigned)((c->n_loc + TILE_N - 1) / TILE_N), (unsigned)(c->kp / c->kb));
+    if (snmf) {
+        if (c->kb == 16) k_gh_posneg_simt<16><<<gg, SIMT_THREADS, 0, c->stream>>>(c->st, c->Gpos, c->Gneg, Hc, c->ldh, c->n_loc, c->kp, c->Dp, c->Dn);
+        else k_gh_posneg_simt<32><<<gg, SIMT_THREADS, 0, c->stream>>>(c->st, c->Gpos, c->Gneg, Hc, c->ldh, c->n_loc, c->kp, c->Dp, c->Dn);
+    } else {
+        if (c->kb == 16) sp::k_gh_simt<16><<<gg, SIMT_THREADS, 0, c->stream>>>(c->st, c->G, Hc, c->ldh, c->n_loc, c->kp, c->GH);
+        else sp::k_gh_simt<32><<<gg, SIMT_THREADS, 0, c->stream>>>(c->st, c->G, Hc, c->ldh, c->n_loc, c->kp, c->GH);
+    }
+    const SparseX& s = c->sx;
+    const float* D = snmf ? c->Dp : c->GH;
+    const float* Dn = snmf ? c->Dn : nullptr;
+    const int kblk = sparse_kblk(c->kp);
+    const int tcol = (sp::SP_THREADS / (kblk / 4)) * sp::SP_COLS_PER_GROUP;
+    dim3 grid((unsigned)((c->n_loc + tcol - 1) / tcol), (unsigned)(c->kp / kblk));
+#define SP_HU(KBLK) sp::k_h_update_csc<KBLK><<<grid, sp::SP_THREADS, 0, c->stream>>>(c->st, s.colptr, s.rowidx, s.vals, \
+        c->W[c->wcur], c->kp, Hc, c->H[c->hcur ^ 1], c->ldh, c->Ht, D, Dn, (float)c->lam_h, c->n_loc)
+    if (kblk == 128) SP_HU(128);
+    else if (kblk == 64) SP_HU(64);
+    else if (kblk == 32) SP_HU(32);
+    else SP_HU(16);
+#undef SP_HU
+    c->launches += 2;
+    CU(cudaGetLastError());
+    return 0;
+}
+
+// Sparse P = [X H^T | H H^T]: H^T (rebuilt if H was set from outside), A panel by panel, B from H^T
+static int launch_xht_sparse(pymfb_ctx* c) {
+    if (c->ht_of != c->hcur) {
+        sp::k_h_transpose<<<grid_for(c->n_loc * c->kp, 256, 16 * c->sm_count), 256, 0, c->stream>>>(c->st, c->H[c->hcur], c->ldh, c->n_loc, c->kp, c->Ht);
+        c->launches += 1;
+        c->ht_of = c->hcur;
+    }
+    const SparseX& s = c->sx;
+    const int kblk = sparse_kblk(c->kp);
+    const int rows_per_cta = sp::SP_THREADS / (kblk / 4);
+    dim3 grid((unsigned)((c->d + rows_per_cta - 1) / rows_per_cta), (unsigned)(c->kp / kblk));
+    for (int p = 0; p < s.npanels; ++p) {
+        const int64_t* rp = s.rowptr + (int64_t)p * c->d;
+#define SP_XHT(KBLK) sp::k_xht_csr<KBLK><<<grid, sp::SP_THREADS, 0, c->stream>>>(c->st, rp, s.ccol, s.cval, c->Ht, c->kp, c->P, c->d, p == 0)
+        if (kblk == 128) SP_XHT(128);
+        else if (kblk == 64) SP_XHT(64);
+        else if (kblk == 32) SP_XHT(32);
+        else SP_XHT(16);
+#undef SP_XHT
+    }
+    dim3 gh((unsigned)((c->kp + TILE_N - 1) / TILE_N), (unsigned)(c->kp / c->kb), (unsigned)c->hh_splits);
+    if (c->kb == 16)
+        k_ltr_partial_simt<16><<<gh, SIMT_THREADS, 0, c->stream>>>(c->st, c->Ht, c->kp, c->Ht, c->kp, c->kp, c->n_loc,
+                                                                   c->hh_rows_per_split, c->hh_part, c->kp, c->kp);
+    else
+        k_ltr_partial_simt<32><<<gh, SIMT_THREADS, 0, c->stream>>>(c->st, c->Ht, c->kp, c->Ht, c->kp, c->kp, c->n_loc,
+                                                                   c->hh_rows_per_split, c->hh_part, c->kp, c->kp);
+    const int64_t cnt = (int64_t)c->kp * c->kp;
+    k_sum_partials<<<(unsigned)((cnt + 255) / 256), 256, 0, c->stream>>>(c->st, c->hh_part, c->hh_splits, cnt, c->P + c->d * c->kp);
+    c->launches += s.npanels + 2;
+    CU(cudaGetLastError());
+    return 0;
+}
+
 // H update pass: H[hcur] -> H[hcur^1]
 static int launch_h_update(pymfb_ctx* c) {
     cudaEvent_t e0, e1;
@@ -386,6 +489,8 @@ static int launch_h_update(pymfb_ctx* c) {
         } else if (c->tc.use_tc2) {
             if (tc2_h_update(c->tc, c->st, c->H[c->hcur], c->H[c->hcur ^ 1], c->stream, &c->launches)) return fail("CTA-pair SS H-update launch failed: %s", cudaGetErrorString(cudaGetLastError()));
         } else if (tc_h_update(c->tc, c->st, c->H[c->hcur], c->H[c->hcur ^ 1], c->stream, &c->launches)) return fail("tcgen05 H-update launch failed: %s", cudaGetErrorString(cudaGetLastError()));
+    } else if (c->path == PYMFB_PATH_SPARSE) {
+        CK(launch_h_update_sparse(c, snmf));
     } else {
         dim3 grid((unsigned)((c->n_loc + TILE_N - 1) / TILE_N), (unsigned)(c->kp / c->kb), (unsigned)c->hsplit);
         if (c->kb == 16)
@@ -404,6 +509,7 @@ static int launch_h_update(pymfb_ctx* c) {
     }
     CK(timing_end(c, 0, e0, e1));
     c->hcur ^= 1;
+    if (c->path == PYMFB_PATH_SPARSE) c->ht_of = c->hcur;     // the sparse H update wrote H^T of the new H
     c->ab_valid = false;
     c->lam_w *= c->inc_w;      // pymf/bnmf.py:84-85: both weights grow at the end of update_h
     c->lam_h *= c->inc_h;
@@ -442,7 +548,8 @@ static void xht_splits(pymfb_ctx* c, int64_t rows, int64_t* cols_per_split, unsi
 static int launch_xht(pymfb_ctx* c) {
     const float* Hc = c->H[c->hcur];
     // deterministic combine (partial copies + ordered sum) overwrites P: nothing to clear
-    const bool overwrite = (c->path == PYMFB_PATH_TC) ? (c->tc.xpart != nullptr) : (c->xpart_simt != nullptr);
+    const bool overwrite = (c->path == PYMFB_PATH_SPARSE) ||
+                           ((c->path == PYMFB_PATH_TC) ? (c->tc.xpart != nullptr) : (c->xpart_simt != nullptr));
     if (!c->p_zeroed && !overwrite) {
         k_zero<<<grid_for(c->ab_count, 256, 8 * c->sm_count), 256, 0, c->stream>>>(c->st, c->P, c->ab_count);
         c->launches += 1;
@@ -452,6 +559,8 @@ static int launch_xht(pymfb_ctx* c) {
     CK(timing_begin(c, 1, &e0, &e1));
     if (c->path == PYMFB_PATH_TC) {
         if (tc_xht(c->tc, c->st, Hc, c->P, c->stream, &c->launches)) return fail("tcgen05 X.H^T launch failed: %s", cudaGetErrorString(cudaGetLastError()));
+    } else if (c->path == PYMFB_PATH_SPARSE) {
+        CK(launch_xht_sparse(c));
     } else {
         // X H^T and H H^T in ONE launch: the row blocks beyond those of X stream H itself
         int64_t cps; unsigned ns;
@@ -483,7 +592,10 @@ static int launch_xht(pymfb_ctx* c) {
 }
 
 static int launch_xx(pymfb_ctx* c) {
-    k_xx<<<XX_BLOCKS, 256, 0, c->stream>>>(c->st, c->X, c->ldx, c->d, c->n_loc, c->red_scratch, c->xps, c->xsh);
+    if (c->sparse)        // the value array as a 1 x nnz row (zero-padded to a multiple of 4)
+        k_xx<<<XX_BLOCKS, 256, 0, c->stream>>>(c->st, c->sx.vals, round_up(c->sx.nnz, 4), 1, c->sx.nnz, c->red_scratch, 0, kNoPanelShift);
+    else
+        k_xx<<<XX_BLOCKS, 256, 0, c->stream>>>(c->st, c->X, c->ldx, c->d, c->n_loc, c->red_scratch, c->xps, c->xsh);
     c->launches += 1;
     CU(cudaGetLastError());
     if (c->world > 1)
@@ -499,7 +611,12 @@ static int launch_err(pymfb_ctx* c, bool store, bool early_stop) {
         const int64_t cnt = c->d * c->kp;
         k_transpose_w<<<(unsigned)((cnt + 255) / 256), 256, 0, c->stream>>>(c->st, c->W[c->wcur], c->d, c->kp, c->Wt, c->ldwt);
         dim3 grid((unsigned)((c->n_loc + TILE_N - 1) / TILE_N), (unsigned)((c->d + c->kb - 1) / c->kb));
-        if (c->kb == 16)
+        const SparseX& s = c->sx;
+        if (c->sparse && c->kb == 16)
+            sp::k_resid_csc<16><<<grid, SIMT_THREADS, 0, c->stream>>>(c->st, s.colptr, s.rowidx, s.vals, c->Wt, c->ldwt, c->H[c->hcur], c->ldh, c->d, c->n_loc, c->kp, c->resid_part);
+        else if (c->sparse)
+            sp::k_resid_csc<32><<<grid, SIMT_THREADS, 0, c->stream>>>(c->st, s.colptr, s.rowidx, s.vals, c->Wt, c->ldwt, c->H[c->hcur], c->ldh, c->d, c->n_loc, c->kp, c->resid_part);
+        else if (c->kb == 16)
             k_resid_simt<16><<<grid, SIMT_THREADS, 0, c->stream>>>(c->st, c->X, c->ldx, c->Wt, c->ldwt, c->H[c->hcur], c->ldh, c->d, c->n_loc, c->kp, c->resid_part, c->xps, c->xsh);
         else
             k_resid_simt<32><<<grid, SIMT_THREADS, 0, c->stream>>>(c->st, c->X, c->ldx, c->Wt, c->ldwt, c->H[c->hcur], c->ldh, c->d, c->n_loc, c->kp, c->resid_part, c->xps, c->xsh);
@@ -547,7 +664,7 @@ static int note_cancellation(pymfb_ctx* c, DevState& hs) {
 
 static int check_ready(pymfb_ctx* c) {
     if (!c) return fail("null context");
-    if (!c->X) return fail("no data bound: call pymfb_bind_x / pymfb_upload_x / pymfb_gen_x first");
+    if (!c->X && !c->sparse) return fail("no data bound: call pymfb_bind_x / pymfb_upload_x / pymfb_upload_x_csc / pymfb_gen_x first");
     if (!c->w_set || !c->h_set) return fail("W and H must be set (pymfb_set_w/h or pymfb_gen_w/h) before running");
     return 0;
 }
@@ -579,7 +696,7 @@ static int enqueue_one(pymfb_ctx* c, bool do_w, bool do_h, bool do_e, bool trace
 }
 
 static LoopState loop_state(const pymfb_ctx* c) {
-    return LoopState{c->wcur, c->hcur, c->ab_valid, c->g_valid, c->xx_valid, c->tc.hs_valid[0], c->tc.hs_valid[1]};
+    return LoopState{c->wcur, c->hcur, c->ab_valid, c->g_valid, c->xx_valid, c->tc.hs_valid[0], c->tc.hs_valid[1], c->ht_of};
 }
 
 static void graph_drop(pymfb_ctx* c) {
@@ -614,7 +731,7 @@ static int graph_build(pymfb_ctx* c, unsigned key, bool do_w, bool do_h, bool do
     const bool periodic = loop_state(c) == s0;
     // capture only recorded the launches: put the scheduling state back to where the stream really is
     c->wcur = s0.wcur; c->hcur = s0.hcur; c->ab_valid = s0.ab; c->g_valid = s0.g; c->xx_valid = s0.xx;
-    c->tc.hs_valid[0] = s0.hs0; c->tc.hs_valid[1] = s0.hs1;
+    c->tc.hs_valid[0] = s0.hs0; c->tc.hs_valid[1] = s0.hs1; c->ht_of = s0.ht;
     if (rc || e != cudaSuccess || !g || !periodic) {
         if (g) cudaGraphDestroy(g);
         cudaGetLastError();
@@ -675,7 +792,7 @@ static int p_unregister(pymfb_ctx* c) {
 // ------------------------------------------------------------------------------------------
 extern "C" {
 
-int pymfb_version(void) { return 1000; }
+int pymfb_version(void) { return 1001; }
 const char* pymfb_last_error(void) { return g_err; }
 
 int pymfb_device_count(void) {
@@ -774,6 +891,7 @@ int pymfb_destroy(pymfb_ctx* c) {
     if (c->comm && c->comm_owned && g_nccl.CommDestroy) g_nccl.CommDestroy(c->comm);
     tc_release(c->tc);
     fused_release(c->fused);
+    sparse_free(c->sx); cudaFree(c->Ht); cudaFree(c->GH); cudaFree(c->hh_part);
     for (int w = 0; w < 2; ++w)
         for (auto& p : c->ev[w]) { cudaEventDestroy(p.first); cudaEventDestroy(p.second); }
     if (c->p_nccl && g_nccl.MemFree) g_nccl.MemFree(c->P); else cudaFree(c->P);
@@ -798,6 +916,8 @@ int pymfb_set_option(pymfb_ctx* c, int option, int64_t value) {
     }
     if (option == PYMFB_OPT_PATH) {
         if (value < 0 || value > 2) return fail("bad path option %lld", (long long)value);
+        if (c->sparse && value != PYMFB_PATH_AUTO)
+            return fail("sparse data runs on its own passes: the dense kernel families (path simt / tc) do not apply");
         c->path_opt = (int)value;
         if (c->X) { CK(resolve_path(c)); if (c->path == PYMFB_PATH_TC) CK(plan_tc(c)); c->g_valid = false; }
         return 0;
@@ -927,6 +1047,17 @@ int pymfb_comm_destroy(void* comm) {
     return 0;
 }
 
+// A dense upload, bind or generator call makes the dense X current again: the sparse buffers go.
+static void sparse_drop(pymfb_ctx* c) {
+    if (!c->sparse) return;
+    cudaStreamSynchronize(c->stream);
+    sparse_free(c->sx);
+    cudaFree(c->Ht); cudaFree(c->GH); cudaFree(c->hh_part);
+    c->Ht = c->GH = c->hh_part = nullptr;
+    c->ht_of = -1;
+    c->sparse = false;
+}
+
 static int data_changed(pymfb_ctx* c) {
     graph_drop(c); c->graph_key = 0;
     if (c->err_auto_switched) { c->err_direct = false; c->err_auto_switched = false; }   // new data: try the identity again
@@ -945,6 +1076,7 @@ static int data_changed(pymfb_ctx* c) {
 // cfg4 k=64 8.44 -> 7.83, cfg5 33.7 -> 31.4, cfg2 1.443 -> 1.405; wider panels (512 .. 16384 columns) gave less.
 // PYMFB_XPANEL=0 keeps everything row-major, =<log2 width> picks another width.
 static int ensure_own_x(pymfb_ctx* c) {
+    sparse_drop(c);
     if (!c->X_own) {
         int sh = 7;
         bool want = (double)c->d * (double)c->n_loc >= 16777216.0 && c->d >= 64 && c->n_loc >= 128 && c->kp % 32 == 0 && c->kp <= 512;
@@ -975,6 +1107,7 @@ int pymfb_bind_x(pymfb_ctx* c, const float* x_dev, int64_t ld) {
     if (ld < c->n_loc || (ld % 4) != 0) return fail("leading dimension %lld must be >= n_local and a multiple of 4", (long long)ld);
     if (((uintptr_t)x_dev & 15) != 0) return fail("x_dev must be 16-byte aligned");
     CU(cudaSetDevice(c->device));
+    sparse_drop(c);
     c->X = x_dev; c->ldx = ld; c->xps = 0; c->xsh = kNoPanelShift;
     return data_changed(c);
 }
@@ -1215,6 +1348,148 @@ int pymfb_upload_x(pymfb_ctx* c, const void* x_host, int dtype, int64_t ld) {
 
 int pymfb_last_upload_pinned(pymfb_ctx* c) { return c && c->last_upload_pinned ? 1 : 0; }
 
+static int factor_stage(pymfb_ctx* c, size_t bytes, void** out);
+
+// ---- sparse X (include/pymfb.h, kernels_sparse.cuh) -----------------------------------------
+// Column-panel CSR of s (CSC on the device): a stable radix sort of the entries by (panel, row) - the entry index is
+// the payload, so a row keeps its column order and the build is deterministic - then the rows' offsets by binary search.
+static int build_csr_panels(pymfb_ctx* c, SparseX& s) {
+    const int64_t d = c->d, n = c->n_loc, nnz = s.nnz;
+    // PYMFB_SPARSE_PANEL (experiment knob): panel width in columns; default: H^T rows of a panel fill ~ half the L2
+    int64_t pw = (int64_t)(63 << 20) / ((int64_t)c->kp * 4);
+    if (const char* e = getenv("PYMFB_SPARSE_PANEL")) { const int64_t v = atoll(e); if (v > 0) pw = v; }
+    s.pw = std::max<int64_t>(1, std::min(pw, n));
+    s.npanels = (int)((n + s.pw - 1) / s.pw);
+    const int64_t nkeys = (int64_t)s.npanels * d;
+    CU(cudaMalloc(&s.rowptr, (size_t)(nkeys + 1) * sizeof(int64_t)));
+    CU(cudaMalloc(&s.ccol, (size_t)std::max<int64_t>(nnz, 1) * sizeof(int32_t)));
+    CU(cudaMalloc(&s.cval, (size_t)std::max<int64_t>(nnz, 1) * sizeof(float)));
+    int32_t* colof = nullptr;
+    uint64_t* keys[2] = {nullptr, nullptr};
+    uint32_t* perm[2] = {nullptr, nullptr};
+    void* temp = nullptr;
+    int rc = 0;
+    auto cleanup = [&]() {
+        cudaStreamSynchronize(c->stream);
+        cudaFree(colof); cudaFree(keys[0]); cudaFree(keys[1]); cudaFree(perm[0]); cudaFree(perm[1]); cudaFree(temp);
+    };
+#define SB(call)                                                                                   \
+    do {                                                                                           \
+        cudaError_t e_ = (call);                                                                   \
+        if (e_ != cudaSuccess) {                                                                   \
+            rc = fail("%s:%d %s -> %s", __FILE__, __LINE__, #call, cudaGetErrorString(e_));        \
+            cleanup();                                                                             \
+            return rc;                                                                             \
+        }                                                                                          \
+    } while (0)
+    const int g = grid_for(std::max<int64_t>(nnz, 1), 256, 16 * c->sm_count);
+    if (nnz > 0) {
+        SB(cudaMalloc(&colof, (size_t)nnz * sizeof(int32_t)));
+        for (int i = 0; i < 2; ++i) {
+            SB(cudaMalloc(&keys[i], (size_t)nnz * sizeof(uint64_t)));
+            SB(cudaMalloc(&perm[i], (size_t)nnz * sizeof(uint32_t)));
+        }
+        sp::k_csc_cols<<<grid_for(n * 32, 256, 16 * c->sm_count), 256, 0, c->stream>>>(s.colptr, n, colof);
+        sp::k_csr_keys<<<g, 256, 0, c->stream>>>(s.rowidx, colof, nnz, d, s.pw, keys[0], perm[0]);
+        SB(cudaGetLastError());
+        int end_bit = 1;
+        while (end_bit < 64 && ((uint64_t)(nkeys - 1) >> end_bit) != 0) ++end_bit;
+        size_t temp_bytes = 0;
+        SB(cub::DeviceRadixSort::SortPairs(nullptr, temp_bytes, keys[0], keys[1], perm[0], perm[1], (int)nnz, 0, end_bit, c->stream));
+        SB(cudaMalloc(&temp, std::max<size_t>(temp_bytes, 16)));
+        SB(cub::DeviceRadixSort::SortPairs(temp, temp_bytes, keys[0], keys[1], perm[0], perm[1], (int)nnz, 0, end_bit, c->stream));
+        sp::k_csr_gather<<<g, 256, 0, c->stream>>>(perm[1], colof, s.vals, nnz, s.ccol, s.cval);
+    }
+    sp::k_csr_rowptr<<<grid_for(nkeys + 1, 256, 16 * c->sm_count), 256, 0, c->stream>>>(keys[1], nnz, nkeys, s.rowptr);
+    c->launches += nnz > 0 ? 5 : 1;
+    SB(cudaGetLastError());
+#undef SB
+    cleanup();
+    return 0;
+}
+
+int pymfb_upload_x_csc(pymfb_ctx* c, const int64_t* colptr, const int32_t* rowidx, const void* values, int dtype, int64_t nnz) {
+    if (!c) return fail("null context");
+    if (!colptr) return fail("colptr is null");
+    if (nnz < 0 || nnz > (int64_t)INT32_MAX) return fail("nnz = %lld: 0 <= nnz < 2^31 supported", (long long)nnz);
+    if (nnz > 0 && (!rowidx || !values)) return fail("rowidx / values are null");
+    if (dtype != PYMFB_F32 && dtype != PYMFB_F64) return fail("bad dtype %d", dtype);
+    if (c->path_opt != PYMFB_PATH_AUTO)
+        return fail("sparse data runs on its own passes: the dense kernel families (path simt / tc) do not apply");
+    CU(cudaSetDevice(c->device));
+    const int64_t n = c->n_loc, nv = round_up(std::max<int64_t>(nnz, 1), 4);
+    SparseX s;
+    s.nnz = nnz;
+    int* flag = nullptr;
+    int bad = 0, rc = 0;
+    auto cleanup = [&]() { cudaStreamSynchronize(c->stream); cudaFree(flag); sparse_free(s); };
+#define SU(call)                                                                                   \
+    do {                                                                                           \
+        cudaError_t e_ = (call);                                                                   \
+        if (e_ != cudaSuccess) {                                                                   \
+            rc = fail("%s:%d %s -> %s", __FILE__, __LINE__, #call, cudaGetErrorString(e_));        \
+            cleanup();                                                                             \
+            return rc;                                                                             \
+        }                                                                                          \
+    } while (0)
+    SU(cudaMalloc(&s.colptr, (size_t)(n + 1) * sizeof(int64_t)));
+    SU(cudaMalloc(&s.rowidx, (size_t)std::max<int64_t>(nnz, 1) * sizeof(int32_t)));
+    SU(cudaMalloc(&s.vals, (size_t)nv * sizeof(float)));
+    SU(cudaMalloc(&flag, sizeof(int)));
+    SU(cudaMemsetAsync(s.vals, 0, (size_t)nv * sizeof(float), c->stream));
+    SU(cudaMemsetAsync(flag, 0, sizeof(int), c->stream));
+    SU(cudaMemcpyAsync(s.colptr, colptr, (size_t)(n + 1) * sizeof(int64_t), cudaMemcpyHostToDevice, c->stream));
+    if (nnz > 0) {
+        SU(cudaMemcpyAsync(s.rowidx, rowidx, (size_t)nnz * sizeof(int32_t), cudaMemcpyHostToDevice, c->stream));
+        if (dtype == PYMFB_F32) {
+            SU(cudaMemcpyAsync(s.vals, values, (size_t)nnz * sizeof(float), cudaMemcpyHostToDevice, c->stream));
+        } else {                                   // fp64 through the factor staging buffer, cast on the device
+            void* stage = nullptr;
+            if ((rc = factor_stage(c, (size_t)nnz * sizeof(double), &stage)) != 0) { cleanup(); return rc; }
+            SU(cudaMemcpyAsync(stage, values, (size_t)nnz * sizeof(double), cudaMemcpyHostToDevice, c->stream));
+            k_cast_in<double><<<grid_for(nnz, 256, 16 * c->sm_count), 256, 0, c->stream>>>((const double*)stage, nnz, s.vals, nnz, 1, nnz);
+            c->launches += 1;
+        }
+    }
+    // the arrays come from outside: no kernel indexes with them before this check has passed
+    sp::k_csc_validate<<<grid_for(n * 32, 256, 16 * c->sm_count), 256, 0, c->stream>>>(s.colptr, s.rowidx, n, nnz, c->d, flag);
+    c->launches += 1;
+    SU(cudaGetLastError());
+    SU(cudaMemcpyAsync(&bad, flag, sizeof(int), cudaMemcpyDeviceToHost, c->stream));
+    SU(cudaStreamSynchronize(c->stream));
+    if (bad) {
+        cleanup();
+        return fail("malformed CSC matrix (%lld x %lld, nnz %lld):%s%s%s%s%s", (long long)c->d, (long long)n, (long long)nnz,
+                    bad & sp::BAD_START ? " colptr[0] != 0;" : "", bad & sp::BAD_PTR_ORDER ? " colptr decreases;" : "",
+                    bad & sp::BAD_END ? " colptr[n] != nnz;" : "", bad & sp::BAD_ROW ? " row index outside [0, d);" : "",
+                    bad & sp::BAD_ROW_ORDER ? " row indices not strictly increasing within a column;" : "");
+    }
+    if ((rc = build_csr_panels(c, s)) != 0) { cleanup(); return rc; }
+    // commit: the sparse X replaces whatever was current
+    sparse_drop(c);
+    if (c->X_own) { CU(cudaFree(c->X_own)); c->X_own = nullptr; }
+    c->X = nullptr;
+    tc_release(c->tc);
+    fused_release(c->fused);
+    c->sx = s;
+    s = SparseX();
+    cudaFree(flag); flag = nullptr;
+    c->sparse = true;
+    c->ht_of = -1;
+    SU(cudaMalloc(&c->Ht, (size_t)n * c->kp * sizeof(float)));
+    SU(cudaMalloc(&c->GH, (size_t)c->kp * c->ldh * sizeof(float)));
+    {   // H H^T row splits: enough CTAs to cover the SMs, >= 64 rows of H^T each
+        const int64_t tiles = ((c->kp + TILE_N - 1) / TILE_N) * (c->kp / c->kb);
+        const int64_t want = std::min<int64_t>(std::max<int64_t>(1, (2LL * c->sm_count) / tiles), std::max<int64_t>(1, n / 64));
+        c->hh_rows_per_split = round_up((n + want - 1) / want, TILE_DK);
+        c->hh_splits = (int)((n + c->hh_rows_per_split - 1) / c->hh_rows_per_split);
+        SU(cudaMalloc(&c->hh_part, (size_t)c->hh_splits * c->kp * c->kp * sizeof(float)));
+    }
+#undef SU
+    c->last_upload_pinned = false;
+    return data_changed(c);
+}
+
 // ---- panel-streamed ingest (include/pymfb.h) --------------------------------------------------
 int pymfb_upload_x_begin(pymfb_ctx* c) {
     if (!c) return fail("null context");
@@ -1419,7 +1694,7 @@ int pymfb_set_w(pymfb_ctx* c, const void* w_host, int dtype) {
 int pymfb_set_h(pymfb_ctx* c, const void* h_host, int dtype) {
     if (!c) return fail("null context");
     CK(set_factor(c, c->H[c->hcur], c->ldh, c->kp, c->k, c->n_loc, h_host, dtype));
-    c->h_set = true; c->ab_valid = false; c->tc.hs_valid[c->hcur] = false;
+    c->h_set = true; c->ab_valid = false; c->tc.hs_valid[c->hcur] = false; c->ht_of = -1;
     return 0;
 }
 int pymfb_get_w(pymfb_ctx* c, void* w_host, int dtype) {
@@ -1449,7 +1724,7 @@ int pymfb_gen_h(pymfb_ctx* c, uint64_t seed) {
     k_gen_uniform<<<grid_for((int64_t)c->k * c->n_loc, 256, 16 * c->sm_count), 256, 0, c->stream>>>(c->H[c->hcur], c->ldh, c->k, c->n_loc, seed, c->n_glob, c->col0);
     c->launches += 1;
     CU(cudaGetLastError());
-    c->h_set = true; c->ab_valid = false; c->tc.hs_valid[c->hcur] = false;
+    c->h_set = true; c->ab_valid = false; c->tc.hs_valid[c->hcur] = false; c->ht_of = -1;
     return 0;
 }
 
@@ -1462,6 +1737,7 @@ static const double kNndsvdTcMinWork = 16777216.0;     // d * n_local
 static const double kNndsvdTcMinWorkWider = 4294967296.0;
 int pymfb_nndsvd(pymfb_ctx* c, int max_iter, double tol, int extra_iter, int* iters_done, double* sigma_out) {
     if (!c) return fail("null context");
+    if (c->sparse) return fail("NNDSVD of sparse data is not supported: upload a dense X");
     if (!c->X) return fail("no data bound: call pymfb_bind_x / pymfb_upload_x / pymfb_gen_x first");
     if (c->world > 1 && !c->comm) return fail("pymfb_nndsvd: world = %d but no communicator is attached", c->world);
     if (max_iter < 1) max_iter = 100;
@@ -1682,6 +1958,7 @@ int pymfb_run(pymfb_ctx* c, int niter, unsigned flags, double* ferr_host, int* n
         c->p_zeroed = false;  // kernels after the stop (incl. the one that clears P) were no-ops
         c->ab_valid = false;
         c->tc.hs_valid[0] = c->tc.hs_valid[1] = false;
+        c->ht_of = -1;
         if (flags & PYMFB_COMPUTE_H) {   // the penalty weights grew once per EXECUTED update_h only
             c->lam_w = lw0; c->lam_h = lh0;
             for (int i = 0; i < done; ++i) { c->lam_w *= c->inc_w; c->lam_h *= c->inc_h; }

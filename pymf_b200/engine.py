@@ -138,7 +138,8 @@ class Engine(object):
 
     @property
     def active_path(self):
-        return {_lib.PATH_SIMT: "simt", _lib.PATH_TC: "tc"}.get(self._lib.pymfb_active_path(self._ctx), "?")
+        return {_lib.PATH_SIMT: "simt", _lib.PATH_TC: "tc",
+                _lib.PATH_SPARSE: "sparse"}.get(self._lib.pymfb_active_path(self._ctx), "?")
 
     @staticmethod
     def comm_unique_id():
@@ -199,6 +200,24 @@ class Engine(object):
             _lib.check(self._lib.pymfb_upload_x_panel(self._ctx, view.ctypes.data_as(C.c_void_p), _dtype_code(view), pw, c0, w, slot))
         _lib.check(self._lib.pymfb_upload_x_end(self._ctx))
         return pw
+
+    def upload_x_csc(self, indptr, indices, values):
+        """Sparse X (d x n_local) in compressed sparse column form: indptr (n_local + 1, int64), indices (row of each
+        non-zero, int32, strictly increasing within a column), values (float32 / float64).  The library checks the
+        arrays before it uses them and raises PymfbError on a malformed matrix.  The context then runs the sparse
+        passes (active_path "sparse") until a dense X is uploaded."""
+        indptr = np.ascontiguousarray(indptr, dtype=np.int64)
+        indices = np.ascontiguousarray(indices, dtype=np.int32)
+        values = np.ascontiguousarray(values)
+        if values.dtype not in (np.float32, np.float64):
+            values = values.astype(np.float64)
+        if indptr.shape != (self.n_local + 1,):
+            raise ValueError("indptr shape %r != (%d,)" % (indptr.shape, self.n_local + 1))
+        if indices.ndim != 1 or values.shape != indices.shape:
+            raise ValueError("indices %r and values %r must be 1-D of the same length" % (indices.shape, values.shape))
+        _lib.check(self._lib.pymfb_upload_x_csc(self._ctx, indptr.ctypes.data_as(C.POINTER(C.c_int64)),
+                                                indices.ctypes.data_as(C.POINTER(C.c_int32)),
+                                                values.ctypes.data_as(C.c_void_p), _dtype_code(values), int(indices.size)))
 
     @property
     def last_upload_pinned(self):

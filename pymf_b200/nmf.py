@@ -12,7 +12,8 @@ Differences that are deliberate and documented in DESIGN.md:
   * X is copied to the GPU on first use and cached (the reference re-reads ``data[:,:]`` on
     every call); assign ``mdl.data = ...`` to replace it;
   * sparse ``data`` is rejected by ``factorize`` (the reference only ever returned the
-    ``-123456`` sentinel for it, :109-112).
+    ``-123456`` sentinel for it, :109-112) unless the object is built with ``sparse=True``: then
+    ``data`` is a scipy.sparse matrix and every call runs the sparse passes of the library.
 """
 import logging
 import sys
@@ -67,6 +68,8 @@ class NMF(object):
       process_group  ``True`` or a ``torch.distributed`` group: ``data`` is this rank's block
                      of COLUMNS, W is replicated, ``.H`` is the local block, ``.ferr`` is global
       path           "auto" | "simt" | "tc"  kernel family (default auto)
+      sparse         ``True``: ``data`` is a 2-D scipy.sparse matrix or array (any format), factorized without
+                     densifying it; ``ferr`` / ``frobenius_norm()`` are the real ||data - W H||
     """
 
     _EPS = 10 ** -8                      # pymf/nmf.py:69
@@ -77,8 +80,14 @@ class NMF(object):
         device = kw.pop("device", None)
         self._pg = kw.pop("process_group", None)
         self._path = kw.pop("path", None)
+        self._sparse = bool(kw.pop("sparse", False))
         if kw:
             raise TypeError("unexpected keyword arguments: %s" % ", ".join(sorted(kw)))
+        if self._sparse:
+            if not _is_sparse(data):
+                raise TypeError("sparse=True needs a scipy.sparse matrix or array as data, got %s" % type(data).__name__)
+            if self._path in ("simt", "tc"):
+                raise ValueError("path=%r names a dense kernel family; sparse data runs on its own passes" % self._path)
 
         def setup_logging():                                   # pymf/nmf.py:73-90
             self._logger = logging.getLogger("pymf")
@@ -194,7 +203,9 @@ class NMF(object):
 
     # ------------------------------------------------------------------ engine
     def _ensure_engine(self):
-        if _is_sparse(self._data):
+        if _is_sparse(self._data) != self._sparse:
+            if self._sparse:
+                raise TypeError("sparse=True needs a scipy.sparse matrix or array as data")
             raise TypeError("sparse data is not supported by the NMF multiplicative-update path")
         if self._engine is None:
             self._engine = self._engine_factory(self._data_dimension, self._n_local, self._num_bases,
@@ -211,6 +222,16 @@ class NMF(object):
 
     def _upload_data(self):
         x = self._data
+        if self._sparse:
+            # canonical CSC of a copy (the caller's matrix is left as it is): duplicates summed, rows sorted
+            m = x.tocsc(copy=True)
+            m.sum_duplicates()
+            if m.shape != (self._data_dimension, self._n_local):
+                raise ValueError("data shape %r != (%d, %d)" % (m.shape, self._data_dimension, self._n_local))
+            vals = m.data if m.data.dtype in (np.float32, np.float64) else m.data.astype(np.float64)
+            self._engine.upload_x_csc(np.ascontiguousarray(m.indptr, dtype=np.int64),
+                                      np.ascontiguousarray(m.indices, dtype=np.int32), np.ascontiguousarray(vals))
+            return
         torch = sys.modules.get("torch")             # a torch.Tensor implies torch is imported; never import it here
         if torch is not None:
             if isinstance(x, torch.Tensor):
@@ -275,8 +296,9 @@ class NMF(object):
 
     # ------------------------------------------------------------------ reference hooks
     def frobenius_norm(self):
-        """||data - W H||_F (pymf/nmf.py:100-114); -123456 if W/H are missing or data is sparse."""
-        if "H" in self._factors and "W" in self._factors and not _is_sparse(self._data):
+        """||data - W H||_F (pymf/nmf.py:100-114); -123456 if W/H are missing, or if data is sparse and the object
+        was not built with sparse=True."""
+        if "H" in self._factors and "W" in self._factors and (self._sparse or not _is_sparse(self._data)):
             return self._sync_to_device().frobenius()
         return _SENTINEL
 

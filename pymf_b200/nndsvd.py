@@ -35,6 +35,8 @@ class NNDSVD(NMF):
     def __init__(self, data, num_bases=4, **kw):
         # path= selects the family of the SVD passes; the engine's own NMF kernels (the error pass) keep their default
         self._svd_path_opt = kw.pop("path", None) or "auto"
+        if kw.get("sparse"):
+            raise TypeError("NNDSVD of sparse data is not supported: pass a dense array")
         super(NNDSVD, self).__init__(data, num_bases, **kw)
 
     @staticmethod
