@@ -81,6 +81,9 @@ __device__ __forceinline__ void tile_mac(float (&acc)[KB / 8][4],
     for (int64_t r0 = r_begin; r0 < r_end; r0 += TILE_DK) {
         const bool has_next = r0 + TILE_DK < r_end;
         if (has_next) load_chunk(r0 + TILE_DK);
+        // each TILE_DK-row step is summed on its own and then added: an fp32 chain of n products carries up to n
+        // roundings, and at k >= 512 (G H) that alone exceeded 1e-5 on small entries (tests/test_elementwise.py)
+        float part[TK][4];
 #pragma unroll
         for (int r = 0; r < TILE_DK; ++r) {
             float4 x = *reinterpret_cast<const float4*>(&Rs[buf][r][tx * 4]);
@@ -89,12 +92,16 @@ __device__ __forceinline__ void tile_mac(float (&acc)[KB / 8][4],
             for (int i = 0; i < TK; ++i) w[i] = Ls[buf][r][ty * TK + i];
 #pragma unroll
             for (int i = 0; i < TK; ++i) {
-                acc[i][0] = fmaf(w[i], x.x, acc[i][0]);
-                acc[i][1] = fmaf(w[i], x.y, acc[i][1]);
-                acc[i][2] = fmaf(w[i], x.z, acc[i][2]);
-                acc[i][3] = fmaf(w[i], x.w, acc[i][3]);
+                part[i][0] = r == 0 ? w[i] * x.x : fmaf(w[i], x.x, part[i][0]);
+                part[i][1] = r == 0 ? w[i] * x.y : fmaf(w[i], x.y, part[i][1]);
+                part[i][2] = r == 0 ? w[i] * x.z : fmaf(w[i], x.z, part[i][2]);
+                part[i][3] = r == 0 ? w[i] * x.w : fmaf(w[i], x.w, part[i][3]);
             }
         }
+#pragma unroll
+        for (int i = 0; i < TK; ++i)
+#pragma unroll
+            for (int j = 0; j < 4; ++j) acc[i][j] += part[i][j];
         if (has_next) store_chunk(buf ^ 1);
         __syncthreads();
         buf ^= 1;
@@ -500,11 +507,12 @@ k_update_w_snmf(const DevState* __restrict__ st, const float* __restrict__ A, co
 //   Wn[i][j] = W[i][j] * A[i][j] / (sum_l W[i][l] B[l][j] + 1e-9)
 // UW_ROWS rows of W per CTA staged in shared memory.  A thread owns ONE column j for a group of UW_RT rows, so that an
 // element B[l][j] (read through L1/L2, coalesced over j) is loaded once per UW_RT outputs and the W values are
-// shared-memory broadcasts (ncu, cold: 80 -> 60 us at 16384 x 128; the W update is ~1 % of a cfg3 step on 8 GPUs).  Every output is still the
-// same sequential fmaf chain over l, so the result is bit-identical to the one-output-per-thread version it replaces.
+// shared-memory broadcasts (ncu, cold: 80 -> 60 us at 16384 x 128; the W update is ~1 % of a cfg3 step on 8 GPUs).  Every output is
+// summed in blocks of UW_SEG terms, the block sums added in order.
 // ---------------------------------------------------------------------------------------
 constexpr int UW_ROWS = 8;      // rows per CTA
 constexpr int UW_RT = 4;        // rows per thread
+constexpr int UW_SEG = 16;      // terms per partial sum of W B
 __global__ void __launch_bounds__(SIMT_THREADS)
 k_update_w(const DevState* __restrict__ st, const float* __restrict__ W, const float* __restrict__ A,
            const float* __restrict__ B, float* __restrict__ Wn, int64_t d, int kp, float lam) {
@@ -521,11 +529,18 @@ k_update_w(const DevState* __restrict__ st, const float* __restrict__ W, const f
         float s[UW_RT];
 #pragma unroll
         for (int r = 0; r < UW_RT; ++r) s[r] = 0.f;
-#pragma unroll 4
-        for (int l = 0; l < kp; ++l) {
-            const float b = __ldg(B + (int64_t)l * kp + j);
+        for (int l0 = 0; l0 < kp; l0 += UW_SEG) {      // blocked sum: one fp32 chain over kp = 512 exceeded 1e-5
+            float t[UW_RT];
 #pragma unroll
-            for (int r = 0; r < UW_RT; ++r) s[r] = fmaf(wr[r * kp + l], b, s[r]);
+            for (int r = 0; r < UW_RT; ++r) t[r] = 0.f;
+#pragma unroll 4
+            for (int l = l0; l < l0 + UW_SEG; ++l) {    // kp is a multiple of UW_SEG
+                const float b = __ldg(B + (int64_t)l * kp + j);
+#pragma unroll
+                for (int r = 0; r < UW_RT; ++r) t[r] = fmaf(wr[r * kp + l], b, t[r]);
+            }
+#pragma unroll
+            for (int r = 0; r < UW_RT; ++r) s[r] += t[r];
         }
 #pragma unroll
         for (int r = 0; r < UW_RT; ++r) {

@@ -132,9 +132,12 @@ k_gh_simt(const DevState* __restrict__ st, const float* __restrict__ G, const fl
         *reinterpret_cast<float4*>(D + (int64_t)(kb0 + ty * TK + i) * ldh + col) = make_float4(acc[i][0], acc[i][1], acc[i][2], acc[i][3]);
 }
 
-// acc += x * row[4 l .. 4 l + 3] over entries [e0, e1) in order; rows of Src (ld floats) picked by idx
-__device__ __forceinline__ void gather_mac(float4& acc, const int32_t* __restrict__ idx, const float* __restrict__ val,
-                                           int64_t e0, int64_t e1, const float* __restrict__ Src, int64_t ld, int off) {
+// acc += x * row[4 l .. 4 l + 3] over entries [e0, e1) in order; rows of Src (ld floats) picked by idx.  The entries
+// are summed in blocks of SP_SEG, the block sums added to acc in order (a single fp32 chain over hundreds of entries
+// carries as many roundings).
+constexpr int SP_SEG = 32;
+__device__ __forceinline__ void gather_mac_seq(float4& acc, const int32_t* __restrict__ idx, const float* __restrict__ val,
+                                               int64_t e0, int64_t e1, const float* __restrict__ Src, int64_t ld, int off) {
     int64_t e = e0;
     for (; e + 4 <= e1; e += 4) {            // four gathers in flight, accumulated in entry order
         float x[4];
@@ -152,6 +155,15 @@ __device__ __forceinline__ void gather_mac(float4& acc, const int32_t* __restric
         const float4 w = *reinterpret_cast<const float4*>(Src + (int64_t)idx[e] * ld + off);
         acc.x = fmaf(x, w.x, acc.x); acc.y = fmaf(x, w.y, acc.y);
         acc.z = fmaf(x, w.z, acc.z); acc.w = fmaf(x, w.w, acc.w);
+    }
+}
+
+__device__ __forceinline__ void gather_mac(float4& acc, const int32_t* __restrict__ idx, const float* __restrict__ val,
+                                           int64_t e0, int64_t e1, const float* __restrict__ Src, int64_t ld, int off) {
+    for (int64_t b = e0; b < e1; b += SP_SEG) {
+        float4 part = make_float4(0.f, 0.f, 0.f, 0.f);
+        gather_mac_seq(part, idx, val, b, min(e1, b + SP_SEG), Src, ld, off);
+        acc.x += part.x; acc.y += part.y; acc.z += part.z; acc.w += part.w;
     }
 }
 

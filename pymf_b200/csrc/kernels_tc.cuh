@@ -2258,15 +2258,16 @@ __global__ void k_split_hilo(const DevState* __restrict__ st, const float* __res
     dst[r * 2 * kpb + kpb + c] = v - hi;
 }
 
-// ---- centering of the small operand (TS kernels, k <= 64) ------------------------------------------------
+// ---- centering of the small operand (TS kernels, k <= 64; PYMFB_CENTER=1, experiments only) ------------------
 // W^T X and G H are sums of POSITIVE products; accumulated with truncation (see "Segments") they come out low
-// by an amount that grows with the chain length.  The TS H-update kernels therefore contract against the
+// by an amount that grows with the chain length.  With PYMFB_CENTER=1 the TS H-update kernels contract against the
 // CENTERED operand W' = W - 1 w_mean^T (column means) resp. G' = G - 1 g_mean^T: the products change sign,
 // the truncation errors stop being one-sided, and the exact identity
 //     W^T x_c = W'^T x_c + w_mean * sum_r x_rc ,     G h_c = G'^T h_c + g_mean * sum_i h_ic
 // is restored in the epilogue with one FMA per output (column sums of X are computed once per data set, those of
 // the H tile come from the registers that already hold it).  Measured on the cfg2 prefix: scale drift of W / H per
-// iteration 1.2e-6 -> see DESIGN.md 5.1.
+// iteration 1.2e-6 -> see DESIGN.md 5.1.  It is off by default: the error of an entry of C becomes
+// eps * w_mean * sum(x) rather than eps * C, which ruins the small entries of parts-based factors.
 constexpr int CM_SPLITS = 64;          // row splits of the column-sum reduction of W
 
 // part[split][c] = sum of src[r][c] over the rows of the split (c < cols <= 64; deterministic order)
@@ -2588,13 +2589,17 @@ inline int tc_plan(TcPlan& p, int device, int sm_count, int64_t d, int64_t n_loc
     p.h_tiles = (int)((n_loc + tc::TILE_COLS - 1) / tc::TILE_COLS);
     { const char* e = getenv("PYMFB_XREV"); p.xrev = (e && e[0] == '1') ? 1 : 0; }
     { const char* e = getenv("PYMFB_SS_PF"); p.ss_pf = e ? std::max(0, atoi(e)) : 0; }
-    {   // Bias of the H-update ratio C / D (see "Segments"): the TS kernels (k <= 64) contract against centered
-        // operands and keep SEG_STAGES-stage segments; the SS kernels give the C chain the D chain's length.
-        // PYMFB_SEG_C / PYMFB_CENTER override both for experiments.
+    {   // Bias of the H-update ratio C / D (see "Segments"): the C chain is kept as short as the D chain (kp / 32
+        // stages).  The TS kernels drain C at least every 2 stages (64 rows, the stage of k_h_update_tsr<KP, 64>, so
+        // that every TS schedule drains at the same rows; k <= 32: 8 MMAs against 4).  The operands stay uncentered: centering
+        // (PYMFB_CENTER=1, experiments only) turns the error of an entry of C into eps * w_mean * sum(x), which on
+        // parts-based data is far larger than the entry itself (tests/test_elementwise.py).
+        // PYMFB_SEG_C overrides the segment length for experiments.
         const char* e = getenv("PYMFB_SEG_C");
         const char* ce = getenv("PYMFB_CENTER");
-        p.center = p.use_ts && !(ce && ce[0] == '0');
-        p.seg_c = (e && atoi(e) > 0) ? atoi(e) : ((p.center || product) ? tc::SEG_STAGES : std::max(1, kp / tc::R1));
+        p.center = p.use_ts && ce && ce[0] == '1';
+        p.seg_c = (e && atoi(e) > 0) ? atoi(e)
+                : ((p.center || product) ? tc::SEG_STAGES : std::max(p.use_ts ? 2 : 1, kp / tc::R1));
         if (p.center) {
             if (cudaMalloc(&p.xsum, (size_t)n_loc * sizeof(float)) != cudaSuccess) { p.err = "cudaMalloc xsum failed"; return 1; }
             if (cudaMalloc(&p.wmean, (size_t)(2 + tc::CM_SPLITS) * kp * sizeof(float)) != cudaSuccess) { p.err = "cudaMalloc wmean failed"; return 1; }

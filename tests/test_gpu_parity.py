@@ -382,6 +382,32 @@ def test_fused_one_pass_kernel_matches_two_pass(shape, monkeypatch):
     assert rel(res["1"][0], res["0"][0]) < 2e-5 and rel(res["1"][1], res["0"][1]) < 2e-5
 
 
+def test_200_iteration_trajectory_on_the_one_pass_kernel():
+    """The one-pass kernel is the default at d <= 256, k <= 32, d n > 2^24 (no knob set here).  Its W^T X chain truncates
+    while its G H (k_gh_ratio) rounds to nearest, so the chain length sets a scale drift per iteration (DESIGN 5.1,
+    "Segments"): W / H must stay within 1e-4 of the float64 oracle over 200 iterations."""
+    d, n, k = 256, 65536 + 128, 32
+    X = O.gen_matrix(81, d, n)
+    W0 = O.gen_matrix(82, d, k).astype(np.float64)
+    H0 = O.gen_matrix(83, k, n).astype(np.float64)
+    Wr, Hr = W0.copy(), H0.copy()
+    e = pymf_b200.Engine(d, n, k)
+    try:
+        e.upload_x(X); e.set_w(W0); e.set_h(H0)
+        e.set_err_mode("trace")
+        at = 0
+        for stop in (50, 100, 200):
+            f, done = e.run(stop - at, early_stop=False)
+            assert done == stop - at
+            O.factorize(X.astype(np.float64), Wr, Hr, niter=stop - at, compute_err=False, early_stop=False)
+            at = stop
+            rw, rh = rel(e.get_w(), Wr), rel(e.get_h(), Hr)
+            assert rw < TOL_WH and rh < TOL_WH, (stop, rw, rh)
+        print("200-iteration one-pass trajectory: rel W %.2e, rel H %.2e" % (rw, rh))
+    finally:
+        e.close()
+
+
 @pytest.mark.parametrize("dtype", [np.float32, np.float64])
 def test_pinned_ingest_equals_pageable_ingest(dtype):
     """X from page-locked memory (direct DMA, pymfb_upload_x fast path) gives the same device
