@@ -163,6 +163,33 @@ int pymfb_upload_x_csc(pymfb_ctx* ctx, const int64_t* colptr /* n_local+1 */, co
                        const void* values, int dtype, int64_t nnz);
 
 /*
+ * Sparse X already on the device, in any order and with duplicates; the library makes the CSC of pymfb_upload_x_csc
+ * from it on the device.
+ *   layout  PYMFB_LAYOUT_COO: a = row ids, b = column ids (nnz each)
+ *           PYMFB_LAYOUT_CSR: a = d + 1 row pointers, b = column ids (nnz)
+ *           PYMFB_LAYOUT_CSC: a = n_local + 1 column pointers, b = row ids (nnz)
+ *   index_dtype PYMFB_I32 / PYMFB_I64 (a and b alike), values nnz entries of dtype PYMFB_F32 / PYMFB_F64.
+ * Every array must be device memory of the context's device (checked with cudaPointerGetAttributes).  The arrays are
+ * checked on the device before any kernel indexes with them - pointers[0] == 0, pointers non-decreasing,
+ * pointers[last] == nnz, 0 <= row < d, 0 <= column < n_local - and a malformed input returns non-zero with the broken
+ * rules in pymfb_last_error(); the context then keeps its previous X.  The canonical form:
+ *   entries sorted by (column, row) with a stable radix sort; the entries of one (row, column) summed in fp64 in
+ *   input order and rounded once to fp32 (explicit zeros are kept, as scipy's sum_duplicates keeps them); int32
+ *   rows strictly increasing within a column, int64 column pointers, fp32 values zero-padded to a multiple of 4.
+ * The same input gives the same arrays on every call.  From there on the call is pymfb_upload_x_csc's (validation,
+ * CSR build, the sparse X becomes current).  It returns after the arrays have been read: the caller may free them
+ * afterwards.  Temporaries: about 24 bytes per input entry plus the CUB sort scratch, freed before returning.
+ * nnz < 2^31.
+ */
+#define PYMFB_LAYOUT_COO 0
+#define PYMFB_LAYOUT_CSR 1
+#define PYMFB_LAYOUT_CSC 2
+#define PYMFB_I32 2
+#define PYMFB_I64 3
+int pymfb_upload_x_sparse_device(pymfb_ctx* ctx, int layout, const void* a, const void* b, int index_dtype,
+                                 const void* values, int dtype, int64_t nnz);
+
+/*
  * Ingest fast path (SURVEY 8f rank 2, the step before the hot path).  pymfb_upload_x looks at
  * its source pointer: PAGE-LOCKED host memory (pymfb_host_alloc, cudaHostAlloc/Register, torch
  * pin_memory) is read by the copy engines directly - fp32 in one strided DMA into X, fp64 in

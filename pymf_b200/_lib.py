@@ -13,6 +13,8 @@ _HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.environ.get("PYMFB_LIB") or os.path.join(_HERE, "libpymfb.so")
 
 F32, F64 = 0, 1
+I32, I64 = 2, 3
+LAYOUT_COO, LAYOUT_CSR, LAYOUT_CSC = 0, 1, 2
 COMPUTE_W, COMPUTE_H, COMPUTE_ERR, EARLY_STOP = 1, 2, 4, 8
 PATH_AUTO, PATH_SIMT, PATH_TC, PATH_SPARSE = 0, 1, 2, 3
 OPT_PATH = 1
@@ -46,6 +48,8 @@ SIGNATURES = {
     "pymfb_upload_x": (C.c_int, [_c_ctx, C.c_void_p, C.c_int, _i64]),
     "pymfb_gen_x": (C.c_int, [_c_ctx, C.c_uint64]),
     "pymfb_upload_x_csc": (C.c_int, [_c_ctx, C.POINTER(_i64), C.POINTER(C.c_int32), C.c_void_p, C.c_int, _i64]),
+    "pymfb_upload_x_sparse_device": (C.c_int, [_c_ctx, C.c_int, C.c_void_p, C.c_void_p, C.c_int, C.c_void_p,
+                                               C.c_int, _i64]),
     "pymfb_host_alloc": (C.c_int, [C.POINTER(C.c_void_p), C.c_size_t]),
     "pymfb_host_free": (C.c_int, [C.c_void_p]),
     "pymfb_last_upload_pinned": (C.c_int, [_c_ctx]),

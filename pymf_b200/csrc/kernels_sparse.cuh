@@ -24,8 +24,8 @@ constexpr int SP_THREADS = 256;
 constexpr int SP_COLS_PER_GROUP = 8;     // columns one lane group contracts in a k_h_update_csc tile
 constexpr int SP_HEAVY = 512;            // a column with more non-zeros is contracted by all groups of the CTA
 
-// pymfb_upload_x_csc validation: bits of the flag
-enum { BAD_START = 1, BAD_PTR_ORDER = 2, BAD_END = 4, BAD_ROW = 8, BAD_ROW_ORDER = 16 };
+// pymfb_upload_x_csc / pymfb_upload_x_sparse_device validation: bits of the flag
+enum { BAD_START = 1, BAD_PTR_ORDER = 2, BAD_END = 4, BAD_ROW = 8, BAD_ROW_ORDER = 16, BAD_COL = 32 };
 
 // One warp per column.  Entries are only read inside [0, nnz) and only for columns whose pointers are ordered.
 __global__ void k_csc_validate(const int64_t* __restrict__ colptr, const int32_t* __restrict__ rowidx, int64_t n,
@@ -91,6 +91,112 @@ __global__ void k_csr_rowptr(const uint64_t* __restrict__ skeys, int64_t nnz, in
             if (skeys[mid] < (uint64_t)k) lo = mid + 1; else hi = mid;
         }
         rowptr[k] = lo;
+    }
+}
+
+// ---------------------------------------------------------------------------------------
+// Device canonicalisation (pymfb_upload_x_sparse_device): a COO, CSR or CSC input with index type T (int32 / int64),
+// in any order and with duplicates, becomes the canonical CSC of pymfb_upload_x_csc.
+//   check    k_sp_check_ptr (CSR / CSC pointers), k_sp_check_idx (every index in range); nothing below runs unless
+//            both passed
+//   keys     key = col * d + row, payload = input position (k_sp_keys_coo, or k_sp_keys_ptr for CSR / CSC)
+//   sort     stable radix sort (sort_pairs in pymfb.cu): duplicates end up adjacent, in input order
+//   runs     k_sp_heads + an in-place inclusive scan give each run of equal keys its output slot; k_sp_sum_runs adds
+//            the run in fp64 in input order and rounds once to fp32 (explicit zeros are kept, as scipy's
+//            sum_duplicates keeps them)
+//   colptr   k_sp_colptr: binary search of c * d in the unique keys
+// ---------------------------------------------------------------------------------------
+// ptr (m + 1 entries): ptr[0] == 0, ptr[m] == nnz, non-decreasing
+template <typename T>
+__global__ void k_sp_check_ptr(const T* __restrict__ ptr, int64_t m, int64_t nnz, int* __restrict__ flag) {
+    const int64_t i0 = (int64_t)blockIdx.x * blockDim.x + threadIdx.x, stride = (int64_t)gridDim.x * blockDim.x;
+    int bad = 0;
+    if (i0 == 0) {
+        if (ptr[0] != 0) bad |= BAD_START;
+        if ((int64_t)ptr[m] != nnz) bad |= BAD_END;
+    }
+    for (int64_t i = i0; i < m; i += stride)
+        if (ptr[i + 1] < ptr[i]) bad |= BAD_PTR_ORDER;
+    if (bad) atomicOr(flag, bad);
+}
+
+// every idx[e] in [0, bound), else `bit`
+template <typename T>
+__global__ void k_sp_check_idx(const T* __restrict__ idx, int64_t nnz, int64_t bound, int bit, int* __restrict__ flag) {
+    const int64_t stride = (int64_t)gridDim.x * blockDim.x;
+    int bad = 0;
+    for (int64_t e = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; e < nnz; e += stride) {
+        const int64_t v = (int64_t)idx[e];
+        if (v < 0 || v >= bound) bad = bit;
+    }
+    if (bad) atomicOr(flag, bad);
+}
+
+template <typename T>
+__global__ void k_sp_keys_coo(const T* __restrict__ rows, const T* __restrict__ cols, int64_t nnz, int64_t d,
+                              uint64_t* __restrict__ keys, uint32_t* __restrict__ perm) {
+    const int64_t stride = (int64_t)gridDim.x * blockDim.x;
+    for (int64_t e = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; e < nnz; e += stride) {
+        keys[e] = (uint64_t)cols[e] * (uint64_t)d + (uint64_t)rows[e];
+        perm[e] = (uint32_t)e;
+    }
+}
+
+// CSR (ptr = d + 1 row pointers, idx = columns) or CSC (ptr = n + 1 column pointers, idx = rows): one warp per row /
+// column.  Only after k_sp_check_ptr has passed: a bad pointer array would write outside keys / perm.
+template <typename T>
+__global__ void k_sp_keys_ptr(const T* __restrict__ ptr, const T* __restrict__ idx, int64_t m, int64_t d, int csc,
+                              uint64_t* __restrict__ keys, uint32_t* __restrict__ perm) {
+    const int lane = threadIdx.x & 31;
+    const int64_t warp = ((int64_t)blockIdx.x * blockDim.x + threadIdx.x) >> 5;
+    const int64_t nwarps = ((int64_t)gridDim.x * blockDim.x) >> 5;
+    for (int64_t o = warp; o < m; o += nwarps)
+        for (int64_t e = (int64_t)ptr[o] + lane; e < (int64_t)ptr[o + 1]; e += 32) {
+            const uint64_t i = (uint64_t)idx[e];
+            keys[e] = csc ? (uint64_t)o * (uint64_t)d + i : i * (uint64_t)d + (uint64_t)o;
+            perm[e] = (uint32_t)e;
+        }
+}
+
+// head[i] = 1 where a run of equal sorted keys starts
+__global__ void k_sp_heads(const uint64_t* __restrict__ skeys, int64_t nnz, uint32_t* __restrict__ head) {
+    const int64_t stride = (int64_t)gridDim.x * blockDim.x;
+    for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < nnz; i += stride)
+        head[i] = (i == 0 || skeys[i] != skeys[i - 1]) ? 1u : 0u;
+}
+
+// One thread per run: the run's values summed in fp64 in input order (the stable sort kept it), rounded once to fp32,
+// stored at slot[i] - 1 (slot = inclusive scan of the heads) with its row and its key.  A run of many duplicates is
+// added by one thread, serially: fine for the few duplicates real data has, slow for a pathological input.
+template <typename V>
+__global__ void k_sp_sum_runs(const uint64_t* __restrict__ skeys, const uint32_t* __restrict__ sperm,
+                              const uint32_t* __restrict__ slot, const V* __restrict__ vals, int64_t nnz, int64_t d,
+                              int32_t* __restrict__ rowidx, float* __restrict__ vout, uint64_t* __restrict__ ukeys) {
+    const int64_t stride = (int64_t)gridDim.x * blockDim.x;
+    for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < nnz; i += stride) {
+        const uint64_t key = skeys[i];
+        if (i > 0 && skeys[i - 1] == key) continue;
+        double s = 0.0;
+        int64_t j = i;
+        do { s += (double)vals[sperm[j]]; ++j; } while (j < nnz && skeys[j] == key);
+        const int64_t o = (int64_t)slot[i] - 1;
+        rowidx[o] = (int32_t)(key % (uint64_t)d);
+        vout[o] = (float)s;
+        ukeys[o] = key;
+    }
+}
+
+// colptr[c] = first unique key >= c * d, c in [0, n]
+__global__ void k_sp_colptr(const uint64_t* __restrict__ ukeys, int64_t nu, int64_t n, int64_t d, int64_t* __restrict__ colptr) {
+    const int64_t stride = (int64_t)gridDim.x * blockDim.x;
+    for (int64_t c = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; c <= n; c += stride) {
+        const uint64_t k = (uint64_t)c * (uint64_t)d;
+        int64_t lo = 0, hi = nu;
+        while (lo < hi) {
+            const int64_t mid = (lo + hi) >> 1;
+            if (ukeys[mid] < k) lo = mid + 1; else hi = mid;
+        }
+        colptr[c] = lo;
     }
 }
 

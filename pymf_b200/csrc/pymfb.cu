@@ -44,6 +44,7 @@
 #include "kernels_sparse.cuh"
 
 #include <cub/device/device_radix_sort.cuh>
+#include <cub/device/device_scan.cuh>
 
 using namespace pymfb;
 
@@ -664,7 +665,7 @@ static int note_cancellation(pymfb_ctx* c, DevState& hs) {
 
 static int check_ready(pymfb_ctx* c) {
     if (!c) return fail("null context");
-    if (!c->X && !c->sparse) return fail("no data bound: call pymfb_bind_x / pymfb_upload_x / pymfb_upload_x_csc / pymfb_gen_x first");
+    if (!c->X && !c->sparse) return fail("no data bound: call pymfb_bind_x / pymfb_upload_x / pymfb_upload_x_csc / pymfb_upload_x_sparse_device / pymfb_gen_x first");
     if (!c->w_set || !c->h_set) return fail("W and H must be set (pymfb_set_w/h or pymfb_gen_w/h) before running");
     return 0;
 }
@@ -792,7 +793,7 @@ static int p_unregister(pymfb_ctx* c) {
 // ------------------------------------------------------------------------------------------
 extern "C" {
 
-int pymfb_version(void) { return 1001; }
+int pymfb_version(void) { return 1002; }
 const char* pymfb_last_error(void) { return g_err; }
 
 int pymfb_device_count(void) {
@@ -1351,6 +1352,21 @@ int pymfb_last_upload_pinned(pymfb_ctx* c) { return c && c->last_upload_pinned ?
 static int factor_stage(pymfb_ctx* c, size_t bytes, void** out);
 
 // ---- sparse X (include/pymfb.h, kernels_sparse.cuh) -----------------------------------------
+// Stable radix sort of (keys[0], perm[0]) into (keys[1], perm[1]) on the bits of keys up to max_key.  Stable: equal
+// keys keep their payload order, so everything built from the result is deterministic.  The CUB scratch is freed
+// before returning (cudaFree waits for the sort).
+static cudaError_t sort_pairs(pymfb_ctx* c, uint64_t* const keys[2], uint32_t* const perm[2], int64_t nnz, uint64_t max_key) {
+    int end_bit = 1;
+    while (end_bit < 64 && (max_key >> end_bit) != 0) ++end_bit;
+    size_t temp_bytes = 0;
+    void* temp = nullptr;
+    cudaError_t e = cub::DeviceRadixSort::SortPairs(nullptr, temp_bytes, keys[0], keys[1], perm[0], perm[1], (int)nnz, 0, end_bit, c->stream);
+    if (e == cudaSuccess) e = cudaMalloc(&temp, std::max<size_t>(temp_bytes, 16));
+    if (e == cudaSuccess) e = cub::DeviceRadixSort::SortPairs(temp, temp_bytes, keys[0], keys[1], perm[0], perm[1], (int)nnz, 0, end_bit, c->stream);
+    cudaFree(temp);
+    return e;
+}
+
 // Column-panel CSR of s (CSC on the device): a stable radix sort of the entries by (panel, row) - the entry index is
 // the payload, so a row keeps its column order and the build is deterministic - then the rows' offsets by binary search.
 static int build_csr_panels(pymfb_ctx* c, SparseX& s) {
@@ -1367,11 +1383,10 @@ static int build_csr_panels(pymfb_ctx* c, SparseX& s) {
     int32_t* colof = nullptr;
     uint64_t* keys[2] = {nullptr, nullptr};
     uint32_t* perm[2] = {nullptr, nullptr};
-    void* temp = nullptr;
     int rc = 0;
     auto cleanup = [&]() {
         cudaStreamSynchronize(c->stream);
-        cudaFree(colof); cudaFree(keys[0]); cudaFree(keys[1]); cudaFree(perm[0]); cudaFree(perm[1]); cudaFree(temp);
+        cudaFree(colof); cudaFree(keys[0]); cudaFree(keys[1]); cudaFree(perm[0]); cudaFree(perm[1]);
     };
 #define SB(call)                                                                                   \
     do {                                                                                           \
@@ -1392,12 +1407,7 @@ static int build_csr_panels(pymfb_ctx* c, SparseX& s) {
         sp::k_csc_cols<<<grid_for(n * 32, 256, 16 * c->sm_count), 256, 0, c->stream>>>(s.colptr, n, colof);
         sp::k_csr_keys<<<g, 256, 0, c->stream>>>(s.rowidx, colof, nnz, d, s.pw, keys[0], perm[0]);
         SB(cudaGetLastError());
-        int end_bit = 1;
-        while (end_bit < 64 && ((uint64_t)(nkeys - 1) >> end_bit) != 0) ++end_bit;
-        size_t temp_bytes = 0;
-        SB(cub::DeviceRadixSort::SortPairs(nullptr, temp_bytes, keys[0], keys[1], perm[0], perm[1], (int)nnz, 0, end_bit, c->stream));
-        SB(cudaMalloc(&temp, std::max<size_t>(temp_bytes, 16)));
-        SB(cub::DeviceRadixSort::SortPairs(temp, temp_bytes, keys[0], keys[1], perm[0], perm[1], (int)nnz, 0, end_bit, c->stream));
+        SB(sort_pairs(c, keys, perm, nnz, (uint64_t)(nkeys - 1)));
         sp::k_csr_gather<<<g, 256, 0, c->stream>>>(perm[1], colof, s.vals, nnz, s.ccol, s.cval);
     }
     sp::k_csr_rowptr<<<grid_for(nkeys + 1, 256, 16 * c->sm_count), 256, 0, c->stream>>>(keys[1], nnz, nkeys, s.rowptr);
@@ -1408,18 +1418,11 @@ static int build_csr_panels(pymfb_ctx* c, SparseX& s) {
     return 0;
 }
 
-int pymfb_upload_x_csc(pymfb_ctx* c, const int64_t* colptr, const int32_t* rowidx, const void* values, int dtype, int64_t nnz) {
-    if (!c) return fail("null context");
-    if (!colptr) return fail("colptr is null");
-    if (nnz < 0 || nnz > (int64_t)INT32_MAX) return fail("nnz = %lld: 0 <= nnz < 2^31 supported", (long long)nnz);
-    if (nnz > 0 && (!rowidx || !values)) return fail("rowidx / values are null");
-    if (dtype != PYMFB_F32 && dtype != PYMFB_F64) return fail("bad dtype %d", dtype);
-    if (c->path_opt != PYMFB_PATH_AUTO)
-        return fail("sparse data runs on its own passes: the dense kernel families (path simt / tc) do not apply");
-    CU(cudaSetDevice(c->device));
-    const int64_t n = c->n_loc, nv = round_up(std::max<int64_t>(nnz, 1), 4);
-    SparseX s;
-    s.nnz = nnz;
+// Shared tail of the sparse uploads.  s holds a CSC X staged on the device (colptr, rowidx, vals, nnz); it is checked
+// before any kernel indexes with it, the column-panel CSR is built from it, and it replaces whatever X was current.
+// s is consumed: freed on failure (the context keeps its previous X), owned by the context on success.
+static int sparse_commit(pymfb_ctx* c, SparseX& s) {
+    const int64_t n = c->n_loc, nnz = s.nnz;
     int* flag = nullptr;
     int bad = 0, rc = 0;
     auto cleanup = [&]() { cudaStreamSynchronize(c->stream); cudaFree(flag); sparse_free(s); };
@@ -1432,25 +1435,8 @@ int pymfb_upload_x_csc(pymfb_ctx* c, const int64_t* colptr, const int32_t* rowid
             return rc;                                                                             \
         }                                                                                          \
     } while (0)
-    SU(cudaMalloc(&s.colptr, (size_t)(n + 1) * sizeof(int64_t)));
-    SU(cudaMalloc(&s.rowidx, (size_t)std::max<int64_t>(nnz, 1) * sizeof(int32_t)));
-    SU(cudaMalloc(&s.vals, (size_t)nv * sizeof(float)));
     SU(cudaMalloc(&flag, sizeof(int)));
-    SU(cudaMemsetAsync(s.vals, 0, (size_t)nv * sizeof(float), c->stream));
     SU(cudaMemsetAsync(flag, 0, sizeof(int), c->stream));
-    SU(cudaMemcpyAsync(s.colptr, colptr, (size_t)(n + 1) * sizeof(int64_t), cudaMemcpyHostToDevice, c->stream));
-    if (nnz > 0) {
-        SU(cudaMemcpyAsync(s.rowidx, rowidx, (size_t)nnz * sizeof(int32_t), cudaMemcpyHostToDevice, c->stream));
-        if (dtype == PYMFB_F32) {
-            SU(cudaMemcpyAsync(s.vals, values, (size_t)nnz * sizeof(float), cudaMemcpyHostToDevice, c->stream));
-        } else {                                   // fp64 through the factor staging buffer, cast on the device
-            void* stage = nullptr;
-            if ((rc = factor_stage(c, (size_t)nnz * sizeof(double), &stage)) != 0) { cleanup(); return rc; }
-            SU(cudaMemcpyAsync(stage, values, (size_t)nnz * sizeof(double), cudaMemcpyHostToDevice, c->stream));
-            k_cast_in<double><<<grid_for(nnz, 256, 16 * c->sm_count), 256, 0, c->stream>>>((const double*)stage, nnz, s.vals, nnz, 1, nnz);
-            c->launches += 1;
-        }
-    }
     // the arrays come from outside: no kernel indexes with them before this check has passed
     sp::k_csc_validate<<<grid_for(n * 32, 256, 16 * c->sm_count), 256, 0, c->stream>>>(s.colptr, s.rowidx, n, nnz, c->d, flag);
     c->launches += 1;
@@ -1488,6 +1474,193 @@ int pymfb_upload_x_csc(pymfb_ctx* c, const int64_t* colptr, const int32_t* rowid
 #undef SU
     c->last_upload_pinned = false;
     return data_changed(c);
+}
+
+int pymfb_upload_x_csc(pymfb_ctx* c, const int64_t* colptr, const int32_t* rowidx, const void* values, int dtype, int64_t nnz) {
+    if (!c) return fail("null context");
+    if (!colptr) return fail("colptr is null");
+    if (nnz < 0 || nnz > (int64_t)INT32_MAX) return fail("nnz = %lld: 0 <= nnz < 2^31 supported", (long long)nnz);
+    if (nnz > 0 && (!rowidx || !values)) return fail("rowidx / values are null");
+    if (dtype != PYMFB_F32 && dtype != PYMFB_F64) return fail("bad dtype %d", dtype);
+    if (c->path_opt != PYMFB_PATH_AUTO)
+        return fail("sparse data runs on its own passes: the dense kernel families (path simt / tc) do not apply");
+    CU(cudaSetDevice(c->device));
+    const int64_t n = c->n_loc, nv = round_up(std::max<int64_t>(nnz, 1), 4);
+    SparseX s;
+    s.nnz = nnz;
+    int rc = 0;
+    auto cleanup = [&]() { cudaStreamSynchronize(c->stream); sparse_free(s); };
+#define SU(call)                                                                                   \
+    do {                                                                                           \
+        cudaError_t e_ = (call);                                                                   \
+        if (e_ != cudaSuccess) {                                                                   \
+            rc = fail("%s:%d %s -> %s", __FILE__, __LINE__, #call, cudaGetErrorString(e_));        \
+            cleanup();                                                                             \
+            return rc;                                                                             \
+        }                                                                                          \
+    } while (0)
+    SU(cudaMalloc(&s.colptr, (size_t)(n + 1) * sizeof(int64_t)));
+    SU(cudaMalloc(&s.rowidx, (size_t)std::max<int64_t>(nnz, 1) * sizeof(int32_t)));
+    SU(cudaMalloc(&s.vals, (size_t)nv * sizeof(float)));
+    SU(cudaMemsetAsync(s.vals, 0, (size_t)nv * sizeof(float), c->stream));
+    SU(cudaMemcpyAsync(s.colptr, colptr, (size_t)(n + 1) * sizeof(int64_t), cudaMemcpyHostToDevice, c->stream));
+    if (nnz > 0) {
+        SU(cudaMemcpyAsync(s.rowidx, rowidx, (size_t)nnz * sizeof(int32_t), cudaMemcpyHostToDevice, c->stream));
+        if (dtype == PYMFB_F32) {
+            SU(cudaMemcpyAsync(s.vals, values, (size_t)nnz * sizeof(float), cudaMemcpyHostToDevice, c->stream));
+        } else {                                   // fp64 through the factor staging buffer, cast on the device
+            void* stage = nullptr;
+            if ((rc = factor_stage(c, (size_t)nnz * sizeof(double), &stage)) != 0) { cleanup(); return rc; }
+            SU(cudaMemcpyAsync(stage, values, (size_t)nnz * sizeof(double), cudaMemcpyHostToDevice, c->stream));
+            k_cast_in<double><<<grid_for(nnz, 256, 16 * c->sm_count), 256, 0, c->stream>>>((const double*)stage, nnz, s.vals, nnz, 1, nnz);
+            c->launches += 1;
+        }
+    }
+#undef SU
+    return sparse_commit(c, s);
+}
+
+// An array pymfb_upload_x_sparse_device reads: device memory of the context's device, aligned to its elements.
+static int check_device_array(const pymfb_ctx* c, const void* p, size_t elem, const char* what) {
+    if (!p) return fail("%s: null pointer", what);
+    if ((uintptr_t)p % elem != 0) return fail("%s: address not aligned to its %zu-byte elements", what, elem);
+    cudaPointerAttributes at;
+    if (cudaPointerGetAttributes(&at, p) != cudaSuccess) { cudaGetLastError(); return fail("%s: not a CUDA pointer", what); }
+    if (at.type != cudaMemoryTypeDevice || at.device != c->device)
+        return fail("%s must be device memory of device %d (memory type %d, device %d)", what, c->device, (int)at.type, at.device);
+    return 0;
+}
+
+// The canonical CSC of a device COO / CSR / CSC input into s (kernels_sparse.cuh, "Device canonicalisation").
+// Temporaries: sort keys and payloads (2 x 12 B per input entry), reused for the run slots and the unique keys, plus
+// the CUB scratch; all freed before returning, after the stream has drained (the caller's arrays have been read).
+extern "C++" {       // a template: C++ linkage inside the extern "C" block
+template <typename T>
+static int sparse_canonical_csc(pymfb_ctx* c, int layout, const T* a, const T* b, const void* values, int dtype,
+                                int64_t nnz, SparseX& s) {
+    const int64_t d = c->d, n = c->n_loc;
+    const int64_t m = layout == PYMFB_LAYOUT_CSR ? d : n;          // pointer array of CSR / CSC: m + 1 entries
+    int* flag = nullptr;
+    uint64_t* keys[2] = {nullptr, nullptr};
+    uint32_t* perm[2] = {nullptr, nullptr};
+    void* temp = nullptr;
+    int bad = 0, rc = 0;
+    auto cleanup = [&]() {
+        cudaStreamSynchronize(c->stream);
+        cudaFree(flag); cudaFree(keys[0]); cudaFree(keys[1]); cudaFree(perm[0]); cudaFree(perm[1]); cudaFree(temp);
+    };
+#define SC(call)                                                                                   \
+    do {                                                                                           \
+        cudaError_t e_ = (call);                                                                   \
+        if (e_ != cudaSuccess) {                                                                   \
+            rc = fail("%s:%d %s -> %s", __FILE__, __LINE__, #call, cudaGetErrorString(e_));        \
+            cleanup();                                                                             \
+            return rc;                                                                             \
+        }                                                                                          \
+    } while (0)
+    const int g = grid_for(std::max<int64_t>(nnz, 1), 256, 16 * c->sm_count);
+    // 1. the arrays come from outside: check them before any kernel indexes with their values
+    SC(cudaMalloc(&flag, sizeof(int)));
+    SC(cudaMemsetAsync(flag, 0, sizeof(int), c->stream));
+    if (layout != PYMFB_LAYOUT_COO) {
+        sp::k_sp_check_ptr<T><<<grid_for(m + 1, 256, 16 * c->sm_count), 256, 0, c->stream>>>(a, m, nnz, flag);
+        c->launches += 1;
+    }
+    if (nnz > 0) {
+        if (layout == PYMFB_LAYOUT_COO) {
+            sp::k_sp_check_idx<T><<<g, 256, 0, c->stream>>>(a, nnz, d, sp::BAD_ROW, flag);
+            c->launches += 1;
+        }
+        const bool rows = layout == PYMFB_LAYOUT_CSC;
+        sp::k_sp_check_idx<T><<<g, 256, 0, c->stream>>>(b, nnz, rows ? d : n, rows ? sp::BAD_ROW : sp::BAD_COL, flag);
+        c->launches += 1;
+    }
+    SC(cudaGetLastError());
+    SC(cudaMemcpyAsync(&bad, flag, sizeof(int), cudaMemcpyDeviceToHost, c->stream));
+    SC(cudaStreamSynchronize(c->stream));
+    if (bad) {
+        static const char* names[3] = {"COO", "CSR", "CSC"};
+        cleanup();
+        return fail("malformed %s matrix (%lld x %lld, nnz %lld):%s%s%s%s%s", names[layout], (long long)d, (long long)n,
+                    (long long)nnz, bad & sp::BAD_START ? " pointers[0] != 0;" : "",
+                    bad & sp::BAD_PTR_ORDER ? " pointers decrease;" : "", bad & sp::BAD_END ? " pointers[last] != nnz;" : "",
+                    bad & sp::BAD_ROW ? " row index outside [0, d);" : "",
+                    bad & sp::BAD_COL ? " column index outside [0, n_local);" : "");
+    }
+    SC(cudaMalloc(&s.colptr, (size_t)(n + 1) * sizeof(int64_t)));
+    int64_t nu = 0;                                                // entries after the duplicates are summed
+    if (nnz > 0) {
+        // 2. (column, row) keys with the input position as payload, 3. stable sort
+        for (int i = 0; i < 2; ++i) {
+            SC(cudaMalloc(&keys[i], (size_t)nnz * sizeof(uint64_t)));
+            SC(cudaMalloc(&perm[i], (size_t)nnz * sizeof(uint32_t)));
+        }
+        if (layout == PYMFB_LAYOUT_COO)
+            sp::k_sp_keys_coo<T><<<g, 256, 0, c->stream>>>(a, b, nnz, d, keys[0], perm[0]);
+        else
+            sp::k_sp_keys_ptr<T><<<grid_for(m * 32, 256, 16 * c->sm_count), 256, 0, c->stream>>>(a, b, m, d, layout == PYMFB_LAYOUT_CSC, keys[0], perm[0]);
+        SC(cudaGetLastError());
+        SC(sort_pairs(c, keys, perm, nnz, (uint64_t)n * (uint64_t)d - 1));
+        // 4. runs of equal keys: heads in perm[0] (free after the sort), scanned in place into 1 + each run's slot
+        uint32_t* slot = perm[0];
+        sp::k_sp_heads<<<g, 256, 0, c->stream>>>(keys[1], nnz, slot);
+        SC(cudaGetLastError());
+        size_t temp_bytes = 0;
+        SC(cub::DeviceScan::InclusiveSum(nullptr, temp_bytes, slot, slot, (int)nnz, c->stream));
+        SC(cudaMalloc(&temp, std::max<size_t>(temp_bytes, 16)));
+        SC(cub::DeviceScan::InclusiveSum(temp, temp_bytes, slot, slot, (int)nnz, c->stream));
+        uint32_t nu32 = 0;
+        SC(cudaMemcpyAsync(&nu32, slot + nnz - 1, sizeof(uint32_t), cudaMemcpyDeviceToHost, c->stream));
+        SC(cudaStreamSynchronize(c->stream));
+        nu = nu32;
+        c->launches += 3;
+    }
+    const int64_t nv = round_up(std::max<int64_t>(nu, 1), 4);
+    SC(cudaMalloc(&s.rowidx, (size_t)std::max<int64_t>(nu, 1) * sizeof(int32_t)));
+    SC(cudaMalloc(&s.vals, (size_t)nv * sizeof(float)));
+    SC(cudaMemsetAsync(s.vals, 0, (size_t)nv * sizeof(float), c->stream));
+    s.nnz = nu;
+    if (nnz > 0) {
+        // sums into the CSC; the unique keys go to keys[0] (free after the sort), 5. column pointers from them
+        if (dtype == PYMFB_F64)
+            sp::k_sp_sum_runs<double><<<g, 256, 0, c->stream>>>(keys[1], perm[1], perm[0], (const double*)values, nnz, d, s.rowidx, s.vals, keys[0]);
+        else
+            sp::k_sp_sum_runs<float><<<g, 256, 0, c->stream>>>(keys[1], perm[1], perm[0], (const float*)values, nnz, d, s.rowidx, s.vals, keys[0]);
+        sp::k_sp_colptr<<<grid_for(n + 1, 256, 16 * c->sm_count), 256, 0, c->stream>>>(keys[0], nu, n, d, s.colptr);
+        c->launches += 2;
+    } else {
+        SC(cudaMemsetAsync(s.colptr, 0, (size_t)(n + 1) * sizeof(int64_t), c->stream));
+    }
+    SC(cudaGetLastError());
+#undef SC
+    cleanup();
+    return 0;
+}
+}  // extern "C++"
+
+int pymfb_upload_x_sparse_device(pymfb_ctx* c, int layout, const void* a, const void* b, int index_dtype,
+                                 const void* values, int dtype, int64_t nnz) {
+    if (!c) return fail("null context");
+    if (layout != PYMFB_LAYOUT_COO && layout != PYMFB_LAYOUT_CSR && layout != PYMFB_LAYOUT_CSC) return fail("bad layout %d", layout);
+    if (index_dtype != PYMFB_I32 && index_dtype != PYMFB_I64) return fail("bad index dtype %d", index_dtype);
+    if (dtype != PYMFB_F32 && dtype != PYMFB_F64) return fail("bad dtype %d", dtype);
+    if (nnz < 0 || nnz > (int64_t)INT32_MAX) return fail("nnz = %lld: 0 <= nnz < 2^31 supported", (long long)nnz);
+    if (c->path_opt != PYMFB_PATH_AUTO)
+        return fail("sparse data runs on its own passes: the dense kernel families (path simt / tc) do not apply");
+    CU(cudaSetDevice(c->device));
+    const size_t isz = index_dtype == PYMFB_I64 ? 8 : 4;
+    if (layout != PYMFB_LAYOUT_COO) CK(check_device_array(c, a, isz, layout == PYMFB_LAYOUT_CSR ? "row pointers" : "column pointers"));
+    if (nnz > 0) {
+        if (layout == PYMFB_LAYOUT_COO) CK(check_device_array(c, a, isz, "row indices"));
+        CK(check_device_array(c, b, isz, layout == PYMFB_LAYOUT_CSC ? "row indices" : "column indices"));
+        CK(check_device_array(c, values, dtype == PYMFB_F64 ? 8 : 4, "values"));
+    }
+    SparseX s;
+    const int rc = index_dtype == PYMFB_I64
+                       ? sparse_canonical_csc<int64_t>(c, layout, (const int64_t*)a, (const int64_t*)b, values, dtype, nnz, s)
+                       : sparse_canonical_csc<int32_t>(c, layout, (const int32_t*)a, (const int32_t*)b, values, dtype, nnz, s);
+    if (rc != 0) { cudaStreamSynchronize(c->stream); sparse_free(s); return rc; }
+    return sparse_commit(c, s);
 }
 
 // ---- panel-streamed ingest (include/pymfb.h) --------------------------------------------------

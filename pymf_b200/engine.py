@@ -219,6 +219,34 @@ class Engine(object):
                                                 indices.ctypes.data_as(C.POINTER(C.c_int32)),
                                                 values.ctypes.data_as(C.c_void_p), _dtype_code(values), int(indices.size)))
 
+    def upload_x_sparse_device(self, layout, a, b, values):
+        """Sparse X (d x n_local) from 1-D torch tensors, canonicalised by the library on the device (entries sorted,
+        duplicates summed; the form is documented at pymfb_upload_x_sparse_device): layout "coo" (a = row ids,
+        b = column ids), "csr" (a = d + 1 row pointers, b = column ids) or "csc" (a = n_local + 1 column pointers,
+        b = row ids).  a and b int32 or int64 alike, values float32 / float64.  CPU tensors are copied to this
+        engine's device (the library refuses memory of another device); torch's current stream there is
+        synchronised before the library reads the arrays, and they are only read during the call."""
+        import torch                                         # already imported: the arguments are torch tensors
+        code = {"coo": _lib.LAYOUT_COO, "csr": _lib.LAYOUT_CSR, "csc": _lib.LAYOUT_CSC}[layout]
+        dev = torch.device("cuda", self.device)
+        a, b, values = ((t.to(dev) if not t.is_cuda else t).contiguous() for t in (a, b, values))
+        torch.cuda.current_stream(dev).synchronize()
+        nnz = int(b.numel())
+        na = {"coo": nnz, "csr": self.d + 1, "csc": self.n_local + 1}[layout]
+        for t, want, what in ((a, na, "a"), (b, nnz, "b"), (values, nnz, "values")):
+            if t.dim() != 1 or t.numel() != want or (want > 1 and t.stride(0) != 1):
+                raise ValueError("%s: expected a contiguous 1-D tensor of %d entries, got shape %r"
+                                 % (what, want, tuple(t.shape)))
+        index = {"torch.int32": _lib.I32, "torch.int64": _lib.I64}
+        if str(a.dtype) not in index or b.dtype != a.dtype:
+            raise TypeError("index tensors must both be int32 or both int64, got %s / %s" % (a.dtype, b.dtype))
+        vcode = {"torch.float32": _lib.F32, "torch.float64": _lib.F64}.get(str(values.dtype))
+        if vcode is None:
+            raise TypeError("values must be float32 or float64, got %s" % values.dtype)
+        _lib.check(self._lib.pymfb_upload_x_sparse_device(self._ctx, code, C.c_void_p(a.data_ptr()),
+                                                          C.c_void_p(b.data_ptr()), index[str(a.dtype)],
+                                                          C.c_void_p(values.data_ptr()), vcode, nnz))
+
     @property
     def last_upload_pinned(self):
         """True if the last upload_x read page-locked memory by direct DMA."""

@@ -13,7 +13,7 @@ Differences that are deliberate and documented in DESIGN.md:
     every call); assign ``mdl.data = ...`` to replace it;
   * sparse ``data`` is rejected by ``factorize`` (the reference only ever returned the
     ``-123456`` sentinel for it, :109-112) unless the object is built with ``sparse=True``: then
-    ``data`` is a scipy.sparse matrix and every call runs the sparse passes of the library.
+    ``data`` is a scipy.sparse matrix or a torch sparse tensor and every call runs the sparse passes of the library.
 """
 import logging
 import sys
@@ -36,6 +36,30 @@ def _is_sparse(a):
         return sp is not None and bool(sp.issparse(a))
     except Exception:
         return False
+
+
+_TORCH_VALUES = ("float16", "bfloat16", "float32", "float64")
+
+
+def _torch_sparse(a):
+    """The torch module if `a` is a torch tensor of a sparse layout, else None (torch is never imported here)."""
+    torch = sys.modules.get("torch")
+    if torch is not None and isinstance(a, torch.Tensor) and a.layout != torch.strided:
+        return torch
+    return None
+
+
+def _check_torch_sparse(t, torch, device):
+    """Raise if the torch sparse tensor `t` cannot be factorized with sparse=True on CUDA device `device` (None: any)."""
+    if t.layout not in (torch.sparse_coo, torch.sparse_csr, torch.sparse_csc):
+        raise TypeError("sparse=True takes torch tensors of layout sparse_coo, sparse_csr or sparse_csc, got %s" % t.layout)
+    if t.dim() != 2 or t.dense_dim() != 0:
+        raise TypeError("sparse=True needs a 2-D torch sparse tensor without batch or dense (hybrid) dimensions, "
+                        "got shape %r with %d dense dimensions" % (tuple(t.shape), t.dense_dim()))
+    if str(t.dtype).replace("torch.", "") not in _TORCH_VALUES:
+        raise TypeError("sparse=True needs float16, bfloat16, float32 or float64 values, got %s" % t.dtype)
+    if device is not None and t.is_cuda and t.device.index != device:
+        raise ValueError("the tensor is on %s but the object computes on cuda:%d; move it there first" % (t.device, device))
 
 
 class _Factor(object):
@@ -68,8 +92,12 @@ class NMF(object):
       process_group  ``True`` or a ``torch.distributed`` group: ``data`` is this rank's block
                      of COLUMNS, W is replicated, ``.H`` is the local block, ``.ferr`` is global
       path           "auto" | "simt" | "tc"  kernel family (default auto)
-      sparse         ``True``: ``data`` is a 2-D scipy.sparse matrix or array (any format), factorized without
-                     densifying it; ``ferr`` / ``frobenius_norm()`` are the real ||data - W H||
+      sparse         ``True``: ``data`` is a 2-D scipy.sparse matrix or array (any format), or a 2-D torch sparse
+                     tensor (``sparse_coo``, coalesced or not, ``sparse_csr`` or ``sparse_csc``; int32 / int64
+                     indices; float16 / bfloat16 / float32 / float64 values; on the CPU or on ``device``),
+                     factorized without densifying it; ``ferr`` / ``frobenius_norm()`` are the real ||data - W H||.
+                     A torch tensor is put into canonical form on the GPU (entries sorted, duplicates summed in
+                     float64 and rounded once to float32); the tensor itself is left as it is
     """
 
     _EPS = 10 ** -8                      # pymf/nmf.py:69
@@ -84,8 +112,12 @@ class NMF(object):
         if kw:
             raise TypeError("unexpected keyword arguments: %s" % ", ".join(sorted(kw)))
         if self._sparse:
-            if not _is_sparse(data):
-                raise TypeError("sparse=True needs a scipy.sparse matrix or array as data, got %s" % type(data).__name__)
+            torch = _torch_sparse(data)
+            if torch is not None:
+                _check_torch_sparse(data, torch, None)                # the device is checked below, once it is known
+            elif not _is_sparse(data):
+                raise TypeError("sparse=True needs a scipy.sparse matrix or array or a torch sparse tensor as data, "
+                                "got %s" % type(data).__name__)
             if self._path in ("simt", "tc"):
                 raise ValueError("path=%r names a dense kernel family; sparse data runs on its own passes" % self._path)
 
@@ -115,6 +147,8 @@ class NMF(object):
             import os
             device = int(os.environ.get("LOCAL_RANK", "0")) if self._pg is not None else 0
         self._device = int(device)
+        if self._sparse and _torch_sparse(data) is not None:
+            _check_torch_sparse(data, _torch_sparse(data), self._device)
 
     # ------------------------------------------------------------------ distributed plumbing
     def _dist(self):
@@ -203,9 +237,10 @@ class NMF(object):
 
     # ------------------------------------------------------------------ engine
     def _ensure_engine(self):
-        if _is_sparse(self._data) != self._sparse:
-            if self._sparse:
-                raise TypeError("sparse=True needs a scipy.sparse matrix or array as data")
+        if self._sparse:
+            if not (_is_sparse(self._data) or _torch_sparse(self._data) is not None):
+                raise TypeError("sparse=True needs a scipy.sparse matrix or array or a torch sparse tensor as data")
+        elif _is_sparse(self._data):
             raise TypeError("sparse data is not supported by the NMF multiplicative-update path")
         if self._engine is None:
             self._engine = self._engine_factory(self._data_dimension, self._n_local, self._num_bases,
@@ -222,6 +257,9 @@ class NMF(object):
 
     def _upload_data(self):
         x = self._data
+        if self._sparse and _torch_sparse(x) is not None:
+            self._upload_torch_sparse(x, _torch_sparse(x))
+            return
         if self._sparse:
             # canonical CSC of a copy (the caller's matrix is left as it is): duplicates summed, rows sorted
             m = x.tocsc(copy=True)
@@ -252,6 +290,22 @@ class NMF(object):
                 return
             x = np.asarray(x)                        # lists / array-likes
         self._engine.upload_x(x)
+
+    def _upload_torch_sparse(self, t, torch):
+        """Hand the index and value arrays of a torch sparse tensor to the library as they are (no coalesce, no
+        layout conversion): it validates them and builds the canonical CSC on the device."""
+        _check_torch_sparse(t, torch, self._device)
+        if tuple(t.shape) != (self._data_dimension, self._n_local):
+            raise ValueError("data shape %r != (%d, %d)" % (tuple(t.shape), self._data_dimension, self._n_local))
+        if t.layout == torch.sparse_coo:
+            layout, a, b, vals = "coo", t._indices()[0], t._indices()[1], t._values()
+        elif t.layout == torch.sparse_csr:
+            layout, a, b, vals = "csr", t.crow_indices(), t.col_indices(), t.values()
+        else:
+            layout, a, b, vals = "csc", t.ccol_indices(), t.row_indices(), t.values()
+        if vals.dtype in (torch.float16, torch.bfloat16):
+            vals = vals.to(torch.float32)                    # exact
+        self._engine.upload_x_sparse_device(layout, a, b, vals)
 
     def _sync_to_device(self):
         eng = self._ensure_engine()
