@@ -174,31 +174,8 @@ __device__ __forceinline__ void mbar_wait_f(uint32_t bar, uint32_t parity, int* 
         if (clock64() - t0 > F_WATCHDOG_CYCLES) f_watchdog(fault, code, aux);
     }
 }
-// TMA load with an L2 eviction-priority hint (createpolicy.fractional.L2::evict_*)
-__device__ __forceinline__ void tma_load_2d_hint(uint32_t dst, const CUtensorMap* map, uint32_t bar, int c0, int c1, uint64_t policy) {
-    asm volatile(
-        "cp.async.bulk.tensor.2d.shared::cluster.global.mbarrier::complete_tx::bytes.L2::cache_hint [%0], [%1, {%3, %4}], [%2], %5;"
-        ::"r"(dst), "l"(map), "r"(bar), "r"(c0), "r"(c1), "l"(policy) : "memory");
-}
-__device__ __forceinline__ uint64_t l2_policy_evict_last() {
-    uint64_t p;
-    asm volatile("createpolicy.fractional.L2::evict_last.b64 %0, 1.0;" : "=l"(p));
-    return p;
-}
-__device__ __forceinline__ uint64_t l2_policy_evict_first() {
-    uint64_t p;
-    asm volatile("createpolicy.fractional.L2::evict_first.b64 %0, 1.0;" : "=l"(p));
-    return p;
-}
-__device__ __forceinline__ void tma_load_2d_hint(uint32_t dst, const CUtensorMap* map, uint32_t bar, int c0, int c1, uint64_t policy);
+// L2 prefetch with an eviction-priority hint (the hinted loads are in kernels_tc.cuh)
 __device__ __forceinline__ void tma_prefetch_2d_hint(const CUtensorMap* map, int c0, int c1, uint64_t policy);
-__device__ __forceinline__ void tma_load_x_hint(uint32_t dst, const CUtensorMap* map, uint32_t bar, int col, int row, int xsh, uint64_t policy) {
-    if (xsh == kNoPanel) { tma_load_2d_hint(dst, map, bar, col, row, policy); return; }
-    const int pn = col >> xsh;
-    asm volatile(
-        "cp.async.bulk.tensor.3d.shared::cluster.global.mbarrier::complete_tx::bytes.L2::cache_hint [%0], [%1, {%3, %4, %5}], [%2], %6;"
-        ::"r"(dst), "l"(map), "r"(bar), "r"(col - (pn << xsh)), "r"(row), "r"(pn), "l"(policy) : "memory");
-}
 __device__ __forceinline__ void tma_prefetch_x_hint(const CUtensorMap* map, int col, int row, int xsh, uint64_t policy) {
     if (xsh == kNoPanel) { tma_prefetch_2d_hint(map, col, row, policy); return; }
     const int pn = col >> xsh;

@@ -142,6 +142,29 @@ __device__ __forceinline__ void tma_prefetch_x(const CUtensorMap* map, int col, 
 __device__ __forceinline__ void tma_prefetch_desc(const CUtensorMap* map) {
     asm volatile("prefetch.tensormap [%0];" ::"l"(map) : "memory");
 }
+// TMA loads with an L2 eviction-priority hint (createpolicy.fractional.L2::evict_*)
+__device__ __forceinline__ uint64_t l2_policy_evict_last() {
+    uint64_t p;
+    asm volatile("createpolicy.fractional.L2::evict_last.b64 %0, 1.0;" : "=l"(p));
+    return p;
+}
+__device__ __forceinline__ uint64_t l2_policy_evict_first() {
+    uint64_t p;
+    asm volatile("createpolicy.fractional.L2::evict_first.b64 %0, 1.0;" : "=l"(p));
+    return p;
+}
+__device__ __forceinline__ void tma_load_2d_hint(uint32_t dst, const CUtensorMap* map, uint32_t bar, int c0, int c1, uint64_t policy) {
+    asm volatile(
+        "cp.async.bulk.tensor.2d.shared::cluster.global.mbarrier::complete_tx::bytes.L2::cache_hint [%0], [%1, {%3, %4}], [%2], %5;"
+        ::"r"(dst), "l"(map), "r"(bar), "r"(c0), "r"(c1), "l"(policy) : "memory");
+}
+__device__ __forceinline__ void tma_load_x_hint(uint32_t dst, const CUtensorMap* map, uint32_t bar, int col, int row, int xsh, uint64_t policy) {
+    if (xsh == kNoPanel) { tma_load_2d_hint(dst, map, bar, col, row, policy); return; }
+    const int pn = col >> xsh;
+    asm volatile(
+        "cp.async.bulk.tensor.3d.shared::cluster.global.mbarrier::complete_tx::bytes.L2::cache_hint [%0], [%1, {%3, %4, %5}], [%2], %6;"
+        ::"r"(dst), "l"(map), "r"(bar), "r"(col - (pn << xsh)), "r"(row), "r"(pn), "l"(policy) : "memory");
+}
 
 __device__ __forceinline__ void tmem_alloc(uint32_t dst_smem, uint32_t ncols) {
     asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(dst_smem), "r"(ncols) : "memory");
@@ -731,7 +754,11 @@ k_xht_tc(const __grid_constant__ CUtensorMap mapX, const __grid_constant__ CUten
         return (c_end - c_begin + 31) / 32;
     };
 
+    // L2 priorities: a box of X is read once per pass (evict_first); the [H_hi ; H_lo] chunks of a column range are
+    // re-read by every row-block CTA of that range (evict_last), so streaming X does not push them out of L2.  Against
+    // the default priority for H, evict_last measured equal on cfg3 and 0.5-1 % faster on cfg4 k = 128 / 512.
     if (warp == 0) {
+        const uint64_t pol_x = l2_policy_evict_first();
         RingPos<Cfg::NX> rx;
         for (int task = blockIdx.x; task < num_tasks; task += gridDim.x) {
             int c_begin;
@@ -741,7 +768,7 @@ k_xht_tc(const __grid_constant__ CUtensorMap mapX, const __grid_constant__ CUten
                 mbar_wait_relaxed(bar.done(rx.s), rx.ph ^ 1);
                 if (elect_one()) {
                     mbar_expect_tx(bar.fullx(rx.s), XSTAGE_BYTES);
-                    tma_load_x(xraw(rx.s), &mapX, bar.fullx(rx.s), c_begin + 32 * ch, row0, xsh);
+                    tma_load_x_hint(xraw(rx.s), &mapX, bar.fullx(rx.s), c_begin + 32 * ch, row0, xsh, pol_x);
                     if (pf > 0 && ch + pf < nch) tma_prefetch_x(&mapX, c_begin + 32 * (ch + pf), row0, xsh);
                 }
                 __syncwarp();
@@ -749,6 +776,7 @@ k_xht_tc(const __grid_constant__ CUtensorMap mapX, const __grid_constant__ CUten
             }
         }
     } else if (warp < NPROD) {
+        const uint64_t pol_h = l2_policy_evict_last();
         RingPos<Cfg::NW> rw;
         DoneLag<Cfg::NX, Cfg::NW> lag;
         uint32_t cnt = 0;
@@ -764,7 +792,7 @@ k_xht_tc(const __grid_constant__ CUtensorMap mapX, const __grid_constant__ CUten
                         mbar_arrive(bar.ready(rw.s));
 #else
                         mbar_expect_tx(bar.ready(rw.s), Cfg::HSTAGE_BYTES);
-                        tma_load_2d(hch(rw.s), &mapH, bar.ready(rw.s), 0, ((c_begin >> 5) + ch) * (2 * KP));   // [H_hi ; H_lo] chunk
+                        tma_load_2d_hint(hch(rw.s), &mapH, bar.ready(rw.s), 0, ((c_begin >> 5) + ch) * (2 * KP), pol_h);   // [H_hi ; H_lo] chunk
 #endif
                     }
                     __syncwarp();
@@ -2053,6 +2081,8 @@ k_xht_ts(const __grid_constant__ CUtensorMap mapX, const __grid_constant__ CUten
     };
 
     if (warp < NPROD) {
+        // No L2 priorities here (unlike k_xht_tc): X evict_first measured neutral, [H_hi ; H_lo] evict_last slower
+        // (cfg5 13.5 -> 13.8 ms, cfg4 k = 64 3.30 -> 3.35 ms per pass; profiles/xht_splits.json, profiles/xht_splits_ts.json)
         int s = 0; uint32_t ph = 0; uint32_t pcnt = 0;   // this warp issues stages pcnt % NPROD == warp
         for (int task = blockIdx.x; task < num_tasks; task += gridDim.x) {
             int c_begin, row0; bool hh;
@@ -2608,7 +2638,10 @@ inline int tc_plan(TcPlan& p, int device, int sm_count, int64_t d, int64_t n_loc
             p.xsum_valid = false;
         }
     }
-    // X H^T tasks: (row block, column range); ~4 tasks per SM, each a multiple of 32 columns
+    // X H^T tasks: (row block, column range); ~4 tasks per SM, each a multiple of 32 columns.  Column ranges are not
+    // capped in length: the row-block CTAs of a range share its [H_hi ; H_lo] chunks through L2, where k_xht_tc keeps
+    // them by loading X evict_first and H evict_last (k_xht_ts measured no gain from either).  Few splits keep the
+    // partial copies within the budget of the ordered combine below (cfg3 on one GPU: 37 splits of 888 chunks, 310 MB).
     p.x_rb = (int)((d + 127) / 128);
     const int64_t chunks = (n_loc + 31) / 32;
     int64_t splits = std::max<int64_t>(1, (4LL * sm_count + p.x_rb - 1) / p.x_rb);
@@ -2616,16 +2649,6 @@ inline int tc_plan(TcPlan& p, int device, int sm_count, int64_t d, int64_t n_loc
         auto gcd = [](int64_t a, int64_t b) { while (b) { int64_t t = a % b; a = b; b = t; } return a; };
         const int64_t m = sm_count / gcd(p.x_rb, sm_count);
         splits = std::max<int64_t>(m, (splits + m / 2) / m * m);
-    }
-    {   // long tasks let the CTAs that share a column range drift apart until the [H_hi ; H_lo] stages they
-        // share fall out of L2 (cfg3 on one GPU: 28 K columns per task ran 50 ms against 23 ms for 8 shards
-        // of 3.5 K columns): cap a task at ~4 K columns, keeping the task count a multiple of the CTA count
-        auto gcd = [](int64_t a, int64_t b) { while (b) { int64_t t = a % b; a = b; b = t; } return a; };
-        const int64_t m = sm_count / gcd(p.x_rb, sm_count);
-        if ((chunks + splits - 1) / splits * 32 > 8192) {
-            const int64_t want = (n_loc + 4095) / 4096;
-            splits = std::max<int64_t>(m, (want + m - 1) / m * m);
-        }
     }
     splits = std::min(splits, chunks);
     // Column ranges are whole segments (SEG_STAGES stages) wherever n allows, for X H^T and H H^T alike: the W update
@@ -2645,7 +2668,7 @@ inline int tc_plan(TcPlan& p, int device, int sm_count, int64_t d, int64_t n_loc
         p.hh_tasks = (int)((chunks + hper - 1) / hper);
     }
     {   // Deterministic combine (bit-reproducible W): partial copies instead of atomics while they stay below 1 GiB
-        // (cfg3 on ONE GPU would need 259 x 8 MiB and keeps the atomics; PYMFB_DETERMINISTIC=1 forces, =0 disables)
+        // (every bench workload fits; PYMFB_DETERMINISTIC=1 forces, =0 disables)
         p.x_splits = p.x_tasks / p.x_rb;
         const size_t bytes = ((size_t)p.x_splits * d * kp + (size_t)p.hh_tasks * kp * kp) * sizeof(float);
         const char* e = getenv("PYMFB_DETERMINISTIC");
